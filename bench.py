@@ -28,6 +28,8 @@ A "step" analyses the next 10 s of every track: K1 k_analyse (framing, FFTs, all
                 bounded samples of the same workload: all cores, one thread, and configs[0] on one thread
 
 `--impl reference` times only that CPU path (all host threads), same metric / config / unit.
+`--dump-outputs DIR` writes the raw and smoothed features of the last timed step (a seeded sample of rows when they are larger
+than DUMP_MAX_ROWS) as finite DIR/*.npy, so that two builds can be compared output for output on the same inputs.
 """
 from __future__ import annotations
 
@@ -48,6 +50,7 @@ WINDOW, HOP, SR = 4096, 1024, 48000.0
 METRIC = "analysed frames/sec"
 UNIT = "frames/s"
 FP32_PEAK_THEORETICAL = 148 * 128 * 2 * 1.965e9 / 1e12       # SMs x lanes x FMA x max SM clock (MEASURED_PEAKS.json sm_max_mhz)
+DUMP_MAX_ROWS = 1 << 18      # --dump-outputs: 2 blocks x (values + classes) x 2^18 rows x 12 fp32 + the fp64 row index = 52.4 MB
 
 
 def algorithmic_bytes_per_frame(hop: int) -> float:
@@ -141,6 +144,32 @@ def measured_peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(out_dir: str, outputs: dict, seed: int = 0):
+    """Write each [T, F, 12] device block of `outputs` as out_dir/<name>.npy, float32 [R, 12]: the same R (track, frame) rows of
+    every block, all of them when T * F <= DUMP_MAX_ROWS, else a sample drawn with `seed`.  rows.npy (float64) holds their
+    index t * F + f in ascending order.  Every file is finite: a non-finite value (flatness overflows to +inf on loud noise, as
+    the reference's does) is written as 0 in <name>.npy and classified in <name>_nonfinite.npy (float32: 0 finite, 1 +inf,
+    -1 -inf, 2 NaN); <name>.npy alone does not tell a 0 from an inf.  The engine carries its per-track state from step to step,
+    so the last step depends on every step before it: dumps are comparable between runs with identical arguments, --warmup and
+    --steps included."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    T, F, nf = next(iter(outputs.values())).shape
+    n = T * F
+    rows = np.arange(n) if n <= DUMP_MAX_ROWS else np.sort(np.random.default_rng(seed).choice(n, DUMP_MAX_ROWS, replace=False))
+    for name, x in outputs.items():
+        flat = x.reshape(n, nf)
+        if len(rows) < n:
+            flat = flat.index_select(0, torch.from_numpy(rows).to(x.device))
+        v = flat.cpu().numpy().astype(np.float32)
+        cls = np.select([np.isnan(v), np.isposinf(v), np.isneginf(v)], [2, 1, -1], 0).astype(np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), np.where(cls == 0, v, np.float32(0)))
+        np.save(os.path.join(out_dir, name + "_nonfinite.npy"), cls)
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -294,13 +323,14 @@ def run_c5(args, fxb200, torch, dist, rank, world, local_rank, dev, fp32_peak):
 def run_realtime(args):
     """BASELINE configs[3] through the C++ harness (tools/rt_latency.cpp, built into feature-extractor_b200/build/)."""
     exe = os.path.join(ROOT, "feature-extractor_b200", "build", "rt_latency")
-    if not os.path.exists(exe):
-        os.makedirs(os.path.dirname(exe), exist_ok=True)
-        lib = os.path.join(ROOT, "feature-extractor_b200", "lib")
-        subprocess.run(["g++", "-O2", "-std=c++17", os.path.join(ROOT, "tools", "rt_latency.cpp"), "-I" + os.path.join(ROOT, "include"),
-                        "-L" + lib, "-lfxb200", "-lpthread", "-Wl,-rpath," + lib, "-o", exe], check=True)
-    r = subprocess.run([exe, "512", "256", f"{args.rt_seconds:g}", "1", "128", "2048"], capture_output=True, text=True,
-                       timeout=args.rt_seconds * 2 + 120)
+    with tempfile.TemporaryDirectory() as tmp:
+        if not os.path.exists(exe):         # the tree may be read-only: a harness build() did not leave is compiled outside it
+            exe = os.path.join(tmp, "rt_latency")
+            lib = os.path.join(ROOT, "feature-extractor_b200", "lib")
+            subprocess.run(["g++", "-O2", "-std=c++17", os.path.join(ROOT, "tools", "rt_latency.cpp"), "-I" + os.path.join(ROOT, "include"),
+                            "-L" + lib, "-lfxb200", "-lpthread", "-Wl,-rpath," + lib, "-o", exe], check=True)
+        r = subprocess.run([exe, "512", "256", f"{args.rt_seconds:g}", "1", "128", "2048"], capture_output=True, text=True,
+                           timeout=args.rt_seconds * 2 + 120)
     try:
         d = json.loads(r.stdout.strip().splitlines()[-1])
     except Exception:
@@ -331,7 +361,10 @@ def main():
     ap.add_argument("--rt-seconds", type=float, default=60.0)
     ap.add_argument("--window", type=int, default=4096, help="exploration only: the headline workload is 4096 / 1024")
     ap.add_argument("--hop", type=int, default=1024)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the features of the last timed step (rank 0's tracks) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global WINDOW, HOP
     WINDOW, HOP = args.window, args.hop
 
@@ -420,6 +453,8 @@ def main():
     eng.profile_enable(False)
     ms_max = max_over_ranks(ms_total)
     value = frames_per_step * world * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"raw": raw, "smooth": smooth})
 
     # ---- the box's concurrent upload ceiling ---------------------------------------------------------------------
     h2d_probe = None

@@ -38,6 +38,7 @@ int main (int argc, char** argv)
     const long special = 6;
     const float special_value = 12345.0f;
     std::atomic<int>  special_phase { 0 };       // 0 active from the start, 1 inactive, 2 active again
+    std::atomic<long> reactivated_at { 0 };      // hops_done[1] when the special track became active again
     std::mutex batch_mutex[2];                   // the engine's per-group batch mutex: consumer batches vs life-cycle calls
 
     auto producer = [&] (long first, long n)
@@ -120,6 +121,7 @@ int main (int argc, char** argv)
             {
                 std::lock_guard<std::mutex> lk (batch_mutex[rings.group_of (special)]);
                 rings.activate (special);
+                reactivated_at.store (hops_done[1].load());
                 special_phase.store (2);
             }
         }
@@ -132,7 +134,11 @@ int main (int argc, char** argv)
     th.emplace_back (poller);
     th.emplace_back (poller);
     th.emplace_back (control);
-    while (hops_done[0].load() < total_hops || hops_done[1].load() < total_hops) std::this_thread::sleep_for (std::chrono::milliseconds (1));
+    // the control thread advances one phase per tick: a fast box can reach total_hops before it has re-activated the special
+    // track, so the run also lasts until the re-activated track has been checked for total_hops / 4 more hops
+    while (hops_done[0].load() < total_hops || hops_done[1].load() < total_hops || special_phase.load() != 2 ||
+           hops_done[1].load() < reactivated_at.load() + total_hops / 4)
+        std::this_thread::sleep_for (std::chrono::milliseconds (1));
     stop.store (true, std::memory_order_release);
     for (long g = 0; g < G; ++g) wake[(size_t) g].signal();
     for (auto& t : th) t.join();

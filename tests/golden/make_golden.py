@@ -1,7 +1,8 @@
 """Generate the golden fixtures in this directory from the REFERENCE ITSELF (oracle/_ref/libfxref.so = the headers
 under /root/reference/Source compiled headless against oracle/juce_shim).  Run in the build container only:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py                 # every fixture, from oracle/_ref
+    python tests/golden/make_golden.py --from-port     # port_vs_reference/ only, from the port (see port_vs_reference)
 
 The fixtures are small .npz files: seeded input (regenerated from oracle_util.make_signal, stored as a checksum
 plus the first samples) and the reference's raw / smoothed feature rows and observable diagnostics.
@@ -56,6 +57,40 @@ def legacy():
     print("legacy", out.shape)
 
 
+def port_vs_reference(from_port: bool = False):
+    """port_vs_reference/: what test_port_equals_reference_on_fresh_seeds (tests/test_oracle.py) and
+    test_port_is_bit_identical_to_the_reference_functions (tests/test_legacy.py) compare the port with, on their own inputs.
+    Written from oracle/_ref.  With --from-port, for a tree where oracle/_ref cannot be built, the port's outputs are written
+    instead and 'source' says so: the port was compared bit for bit with oracle/_ref on these inputs while the reference was
+    available, and both tests check the record against oracle/_ref wherever it is built."""
+    from test_legacy import CASES as LEGACY_CASES, signal
+    from test_oracle import FRESH_SEED_CASES, fresh_seed_audio
+
+    ora = ou.port() if from_port else ou.reference()
+    if ora is None:
+        raise SystemExit("oracle/_ref/libfxref.so missing (--from-port records the port's outputs instead)")
+    lib = ou.PORT_SO if from_port else ou.REF_SO
+    out_dir = os.path.join(HERE, "port_vs_reference")
+    os.makedirs(out_dir, exist_ok=True)
+    d = {"source": np.array(ora.kind)}
+    for i, (N, H, sr) in enumerate(FRESH_SEED_CASES):
+        audio = fresh_seed_audio(N, H, sr)
+        r = ora.analyse(audio, window=N, hop=H, sample_rate=sr)
+        d.update({f"c{i}_audio_sum": audio.astype(np.float64).sum(axis=1), f"c{i}_raw": r["raw"], f"c{i}_smooth": r["smooth"],
+                  f"c{i}_lag": r["diag"][..., ou.D["lag"]]})
+    np.savez_compressed(os.path.join(out_dir, "fresh_seeds.npz"), **d)
+    d = {"source": np.array(ora.kind)}
+    for i, (N, sr, sec, F, track) in enumerate(LEGACY_CASES):
+        out, la = ou.legacy_analyse(lib, signal(N, sr, sec, track), F, N, sr)
+        d.update({f"c{i}_out": out[..., :11], f"c{i}_log_attack": la})
+    np.savez_compressed(os.path.join(out_dir, "legacy_cases.npz"), **d)
+    print("port_vs_reference from", ora.kind)
+
+
 if __name__ == "__main__":
-    main()
-    legacy()
+    if "--from-port" in sys.argv:
+        port_vs_reference(from_port=True)
+    else:
+        main()
+        legacy()
+        port_vs_reference()
