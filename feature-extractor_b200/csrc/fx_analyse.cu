@@ -379,7 +379,12 @@ __device__ __noinline__ void fft_core (V16 io, int m0)
 static_assert (3 * (sizeof (Smem<16>) + 1024) <= 233472, "three CTAs of N = 4096 per SM");
 static_assert (FX_CTAS_R8 * (sizeof (Smem<8>) + 1024) <= 233472, "resident CTAs of N = 2048 per SM");
 static_assert (FX_CTAS_R4 * (sizeof (Smem<4>) + 1024) <= 233472, "resident CTAs of N = 1024 per SM");
-template <int R1, bool MG>
+// SP: power-spectrum mode (FX_SPECTRUM_POWER).  Each of the three spectra is handed on as (|X[k]|, 0) instead of
+// (Re X[k], Im X[k]): |B| to the spectral passes and the previous spectrum, P = |C|^2 to FFT-beta, |A| to the harmonic
+// pass.  Everything downstream squares or compares these values exactly as it squares and compares Re, so the two
+// places that form them (the split after FFT-alpha, the hand-over of A after FFT-beta) are the only branches on SP;
+// the instantiations without it are the parity mode, unchanged.
+template <int R1, bool MG, bool SP>
 __global__ void __launch_bounds__ (16 * R1, (R1 == 16 ? 3 : (R1 == 8 ? FX_CTAS_R8 : FX_CTAS_R4)))
 k_analyse (const AnalyseParams p)
 {
@@ -629,6 +634,7 @@ k_analyse (const AnalyseParams p)
         //   Re B = (Zk.x + Zn.x) / 2   Im B = (Zk.y - Zn.y) / 2   Re C = (Zk.y + Zn.y) / 2     (the buffer holds Z / 2)
         // Re B stays in registers for the spectral passes; P[k] = Re C[k]^2 (PitchAnalyser.h:97-104, imaginary part
         // cleared) goes to the P / Re A array as the imaginary input of FFT-beta.
+        // Power mode (SP): |B| takes Re B's place, Im C = (Re Z[N-k] - Re Z[k]) / 2 and P = |C|^2.
         float cr[8];
         float rawmax = 0.0f;     // SpectralCharacteristics.h:153: max |buf[j]|, j < M, over the interleaved Re/Im floats = bins k < M/2
         float psum = 0.0f;       // sum of P^2 over the lower half: sets the power-of-two scale P is transformed at
@@ -641,9 +647,19 @@ k_analyse (const AnalyseParams p)
                 const float2 zn = sm.ex[j == 0 ? zb_self : zb_mirror + zrun<R1> (8 - j)];      // Z[(N - k) & (N - 1)]
                 const float reB = zk.x + zn.x, reC = zk.y + zn.y;
                 const float imB = zk.y - zn.y;
-                cr[j] = reB;
-                if (b0 < M / 2) rawmax = fmaxf (rawmax, fmaxf (fabsf (reB), fabsf (imB)));
-                pq[j] = __fmul_rn (reC, reC);
+                if (SP)
+                {
+                    const float imC = zn.x - zk.x;
+                    cr[j] = __fsqrt_rn (fmaf (reB, reB, __fmul_rn (imB, imB)));
+                    if (b0 < M / 2) rawmax = fmaxf (rawmax, cr[j]);                              // the odd (Im) slots hold 0
+                    pq[j] = fmaf (reC, reC, __fmul_rn (imC, imC));
+                }
+                else
+                {
+                    cr[j] = reB;
+                    if (b0 < M / 2) rawmax = fmaxf (rawmax, fmaxf (fabsf (reB), fabsf (imB)));
+                    pq[j] = __fmul_rn (reC, reC);
+                }
                 psum = fmaf (pq[j], pq[j], psum);
             }
             *reinterpret_cast<float4*> (&sm.pa[pb0])     = make_float4 (pq[0], pq[1], pq[2], pq[3]);
@@ -996,11 +1012,21 @@ k_analyse (const AnalyseParams p)
                 runf += av[j];
             }
 #endif
-            // Re A of this thread's 8 bins moves to the P / Re A array (P was consumed by the transform)
+            // Re A of this thread's 8 bins moves to the P / Re A array (P was consumed by the transform).  Power mode: |A|, with
+            // Im A[k] = (Im Z[k] - Im Z[N-k]) / 2 -- Im A is odd and 2^k D even, so D cancels.
             {
                 float ra[8];
                 #pragma unroll
-                for (int j = 0; j < 8; ++j) ra[j] = sm.ex[zb_own + zrun<R1> (j)].x;
+                for (int j = 0; j < 8; ++j)
+                {
+                    if (SP)
+                    {
+                        const float2 zk = sm.ex[zb_own + zrun<R1> (j)];
+                        const float imA = 0.5f * (zk.y - sm.ex[j == 0 ? zb_self : zb_mirror + zrun<R1> (8 - j)].y);
+                        ra[j] = __fsqrt_rn (fmaf (zk.x, zk.x, __fmul_rn (imA, imA)));
+                    }
+                    else ra[j] = sm.ex[zb_own + zrun<R1> (j)].x;
+                }
                 *reinterpret_cast<float4*> (&sm.pa[pb0])     = make_float4 (ra[0], ra[1], ra[2], ra[3]);
                 *reinterpret_cast<float4*> (&sm.pa[pb0 + 4]) = make_float4 (ra[4], ra[5], ra[6], ra[7]);
             }
@@ -1693,18 +1719,30 @@ template <int R1> static cudaError_t launch_t (long n_tracks, const AnalyseParam
 {
     const long grid = n_tracks * p.n_chunks;
     if (grid <= 0) return cudaSuccess;
-    if (p.want_margins) k_analyse<R1, true><<<(unsigned) grid, 16 * R1, sizeof (Smem<R1>), stream>>> (p);
-    else                k_analyse<R1, false><<<(unsigned) grid, 16 * R1, sizeof (Smem<R1>), stream>>> (p);
+    const unsigned g = (unsigned) grid, nt = 16 * R1;
+    const size_t smem = sizeof (Smem<R1>);
+    if (p.spectrum == FX_SPECTRUM_POWER)
+    {
+        if (p.want_margins) k_analyse<R1, true, true><<<g, nt, smem, stream>>> (p);
+        else                k_analyse<R1, false, true><<<g, nt, smem, stream>>> (p);
+    }
+    else
+    {
+        if (p.want_margins) k_analyse<R1, true, false><<<g, nt, smem, stream>>> (p);
+        else                k_analyse<R1, false, false><<<g, nt, smem, stream>>> (p);
+    }
     return cudaGetLastError();
 }
 
 template <int R1> static cudaError_t configure_t()
 {
-    cudaError_t ce = cudaFuncSetAttribute (k_analyse<R1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sizeof (Smem<R1>));
-    if (ce != cudaSuccess) return ce;
-    ce = cudaFuncSetAttribute (k_finalize<R1 / 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (kFzBufs * 32 * frame_rec_bytes (256 * R1)));
-    if (ce != cudaSuccess) return ce;
-    return cudaFuncSetAttribute (k_analyse<R1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sizeof (Smem<R1>));
+    const int smem = (int) sizeof (Smem<R1>);
+    cudaError_t ce = cudaFuncSetAttribute (k_finalize<R1 / 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (kFzBufs * 32 * frame_rec_bytes (256 * R1)));
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    return ce;
 }
 
 int analyse_ctas_per_sm (int window)

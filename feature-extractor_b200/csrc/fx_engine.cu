@@ -279,6 +279,7 @@ fx_status run_range (fx_engine* e, int t0, int nt, int n_chunks, int flip, long 
     for (int k = 0; k < 16; ++k) a.f0bin_pow2[k] = e->f0bin_pow2[k];
     a.rec = sc.rec;
     a.first_spec = sc.first_spec; a.last_spec = sc.last_spec; a.first_idx = sc.first_idx;
+    a.spectrum = e->cfg.spectrum;
     const bool prof = may_profile && e->profiling;
     fx_engine::ProfRec pr{};
     if (prof)
@@ -600,6 +601,7 @@ void fx_default_config (fx_config* c)
     c->max_frames_per_call = 0;       // grow on demand
     c->ring_hops = 16;
     c->tracks_per_group = 0;
+    c->spectrum = FX_SPECTRUM_RE_SQUARED;   // the reference's Re(X)^2
 }
 
 const char* fx_version (void) { return "fxb200 0.2 (sm_100a)"; }
@@ -618,6 +620,7 @@ fx_status fx_engine_create (const fx_config* cfg, fx_engine** out)
     if (cfg->rms_pushes_per_frame != 1 && cfg->rms_pushes_per_frame != 2) { g_create_error = "rms_pushes_per_frame must be 1 or 2"; return FX_ERR_INVALID_ARG; }
     if (cfg->ring_hops < 0 || cfg->tracks_per_group < 0) { g_create_error = "ring_hops and tracks_per_group must be >= 0"; return FX_ERR_INVALID_ARG; }
     if (! (cfg->sample_rate > 0.0)) { g_create_error = "sample_rate must be positive"; return FX_ERR_INVALID_ARG; }
+    if (cfg->spectrum != FX_SPECTRUM_RE_SQUARED && cfg->spectrum != FX_SPECTRUM_POWER) { g_create_error = "spectrum must be FX_SPECTRUM_RE_SQUARED or FX_SPECTRUM_POWER"; return FX_ERR_INVALID_ARG; }
 
     int ndev = 0;
     if (cudaGetDeviceCount (&ndev) != cudaSuccess || ndev == 0) { g_create_error = "no CUDA device (this library has no CPU fallback)"; return FX_ERR_NO_DEVICE; }

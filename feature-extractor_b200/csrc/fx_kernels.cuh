@@ -92,9 +92,10 @@ struct AnalyseParams
     short        f0bin_pow2[16];   // her_tab[lag][18] for lag = 2^k (the lags whose f0 bin the kernel does not derive by integer division)
     // outputs
     unsigned char* rec;            // [n_tracks][n_frames] records of frame_rec_bytes (window) each
-    float*       first_spec;       // [n_tracks][n_chunks][M]  Re spectrum (windowed path) of the chunk's first non-silent frame
+    float*       first_spec;       // [n_tracks][n_chunks][M]  Re (power mode: |X|) spectrum (windowed path) of the chunk's first non-silent frame
     float*       last_spec;        // [n_tracks][n_chunks][M]  ... of its last non-silent frame
     int*         first_idx;        // [n_tracks][n_chunks]     frame index of the first non-silent frame, -1 if none
+    int          spectrum;         // fx_config::spectrum: FX_SPECTRUM_RE_SQUARED or FX_SPECTRUM_POWER (selects the instantiation)
 };
 
 int         analyse_ctas_per_sm (int window);      // resident CTAs per SM k_analyse is compiled for (chunk heuristic)
@@ -122,7 +123,7 @@ struct FluxFixParams
     const float* first_spec;
     const float* last_spec;
     const int*   first_idx;
-    const float* prev_in;          // [n_tracks][M] carried "previousBinMagnitudes" as Re values (zeros after reset)
+    const float* prev_in;          // [n_tracks][M] carried "previousBinMagnitudes" as Re values, |X| in power mode (zeros after reset)
     float*       prev_out;
     float*       raw;
 };

@@ -49,12 +49,17 @@ class Config(ctypes.Structure):
         ("n_tracks", c_int), ("window", c_int), ("hop", c_int), ("sample_rate", c_double), ("device", c_int),
         ("rms_pushes_per_frame", c_int), ("onset_type", c_int), ("onset_hist", c_int), ("onset_multiplier", c_float),
         ("gain", c_float), ("max_frames_per_call", c_long), ("ring_hops", c_int), ("tracks_per_group", c_int),
+        ("spectrum", c_int),
     ]
 
 
 class RtStats(ctypes.Structure):
     _fields_ = [("batches", c_uint64), ("hops", c_uint64), ("overruns", c_uint64), ("batch_ms_mean", c_double), ("batch_ms_max", c_double)]
 
+
+# fx_config.spectrum (fx_engine.h FX_SPECTRUM_*): the reference's Re(X)^2 per bin (default), or |X|^2 -- Engine(spectrum=SPECTRUM_POWER)
+SPECTRUM_RE_SQUARED = 0
+SPECTRUM_POWER = 1
 
 FEATURES_CALLBACK = ctypes.CFUNCTYPE(None, c_void_p, c_int, c_int, c_uint64, c_int)
 

@@ -93,10 +93,12 @@ public:
     struct AudioDeviceSetup { int bufferSize = 512; double sampleRate = 48000.0; };
 
     AudioDeviceManager (int numInputChannels, double sampleRate = 48000.0, int bufferSize = 512,
-                        int windowSize = 2048, int device = 0, int tracksPerGroup = 0)
+                        int windowSize = 2048, int device = 0, int tracksPerGroup = 0,
+                        int spectrum = FX_SPECTRUM_RE_SQUARED)       // FX_SPECTRUM_POWER: |X|^2 per bin (fx_engine.h)
     {
         fx_config cfg;
         fx_default_config (&cfg);
+        cfg.spectrum = spectrum;
         cfg.n_tracks = numInputChannels;
         cfg.window = windowSize;                 // AnalyserTrackController.h:20-21
         cfg.hop = windowSize / 2;                // RealTimeAudioAnalysis.h:207

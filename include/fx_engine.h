@@ -63,6 +63,21 @@ enum {
 #define FX_OSC_FLOATS_CODE   12
 #define FX_OSC_FLOATS_README 10
 
+/* Spectrum mode (fx_config.spectrum).  The reference squares only the REAL part of each FFT bin wherever it reads a spectrum
+ * (SpectralCharacteristics.h:68-73, :158-159; HarmonicCharacteristics.h:63-64; PitchAnalyser.h:100-103), so its features
+ * depend on the phase at which the hop meets the signal: a steady tone makes the harmonic energy ratio, inharmonicity,
+ * flatness and slope flicker over their whole range.
+ *   FX_SPECTRUM_RE_SQUARED  the reference's values (parity mode, the default).
+ *   FX_SPECTRUM_POWER       each of the three forward transforms per hop hands its consumers (|X[k]|, 0) in place of
+ *                           (Re X[k], Im X[k]), k = 0 .. N-1, |X| = (float) sqrt ((double) Re^2 + (double) Im^2) (the GPU
+ *                           forms it in fp32).  Nothing else changes, so the reference's own code defines the result: the
+ *                           per-bin value of the spectral features, flux, flatness, slope and harmonic features becomes
+ *                           |X|^2; the pitch path's P[k] becomes |C[k]|^2, whose inverse transform is then the true circular
+ *                           autocorrelation; the slope's pre-max scans |X[k]| for k < N/4; the previous spectrum holds |X|.
+ * The mode applies to every analysis path (fx_analyse_host / _device / _host_pcm and the real-time workers); the legacy
+ * analyser is unaffected (it already uses true magnitudes).  fx_engine_create refuses any other value. */
+enum { FX_SPECTRUM_RE_SQUARED = 0, FX_SPECTRUM_POWER = 1 };
+
 typedef struct fx_config {
     int    n_tracks;            /* one AnalyserTrackController per track (AnalyserTrackController.h:17) */
     int    window;              /* N: 1024, 2048 (reference: AnalyserTrackController.h:20-21) or 4096 */
@@ -77,7 +92,10 @@ typedef struct fx_config {
     long   max_frames_per_call; /* capacity of the engine-owned device result buffers (frames per track per call) */
     int    ring_hops;           /* streaming: device + pinned ring length in hops per track (>= window/hop + 2); 0 = no real-time path */
     int    tracks_per_group;    /* streaming: tracks per CUDA stream / pinned-ring group; 0 = all tracks in one group */
+    int    spectrum;            /* FX_SPECTRUM_*: what every spectrum consumer reads per bin; fixed for the engine's life */
 } fx_config;
+/* NOTE: fx_config grew by the trailing `spectrum` field.  Always fill it with fx_default_config (never a hand-sized
+ * copy): a caller compiled against the older, shorter struct has fx_default_config write past its end. */
 
 void        fx_default_config (fx_config* cfg);
 

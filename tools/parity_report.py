@@ -16,6 +16,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [os.path.join(ROOT, "feature-extractor_b200"), os.path.join(ROOT, "tests")]
 import fxb200
 import oracle_util as ou
+import power_oracle
 
 
 def engine_offline(audio, N, H, sr, **kw):
@@ -63,12 +64,15 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "parity.json"))
     ap.add_argument("--quick", action="store_true", help="short streams (a smoke run of this script)")
+    ap.add_argument("--spectrum", choices=("re2", "power"), default="re2",
+                    help="power: only the configs[1] shape, the engine in power-spectrum mode (fx_config.spectrum = 1) against "
+                         "tests/power_oracle.py")
     args = ap.parse_args()
-    ora = ou.best_oracle()
+    ora = ou.best_oracle() if args.spectrum == "re2" else power_oracle.CheckedPowerOracle()
     q = args.quick
     report = {"oracle": ora.kind, "tolerance": ou.TOL, "margin_tolerance": ou.MARGIN_TOL,
               "rule": "a mismatch is exempt only when the ORACLE's decision margin (port side) is below margin_tolerance; GPU margins are diagnostic",
-              "configs": {}}
+              "spectrum": args.spectrum, "configs": {}}
 
     def add(name, what, g, o, extra=None):
         res = ou.compare(g, o)
@@ -78,6 +82,19 @@ def main():
             res.update(extra)
         report["configs"][name] = res
         print(name, ou.summary(res), flush=True)
+
+    if args.spectrum == "power":
+        # |X|^2 per bin (fx_engine.h FX_SPECTRUM_POWER) at the configs[1] shape: the one full-size leg of the mode
+        N, H, sr = 2048, 512, 48000.0
+        a = ou.make_tracks(8 if q else 64, (5 if q else 60) * 48000 // H * H, sr)
+        add("c2_power", f"configs[1] shape in power-spectrum mode: {a.shape[0]} tracks x {a.shape[1] / sr:g} s, N=2048 H=512",
+            engine_offline(a, N, H, sr, spectrum=fxb200.SPECTRUM_POWER), power_oracle.CheckedPowerOracle().analyse(a, window=N, hop=H, sample_rate=sr))
+        c = report["configs"]["c2_power"]
+        report["totals"] = {k: c[k] for k in ("frames", "raw_mismatch_total", "raw_mismatch_exempt", "bad_raw", "lag_mismatch", "bad_lag", "bad_smooth",
+                                              "gpu_only_low_margin_frames", "exempt_by_cause", "max_abs_err")}
+        os.makedirs(os.path.dirname(args.out), exist_ok=True)
+        json.dump(report, open(args.out, "w"), indent=1)
+        sys.exit(0 if c["bad_raw"] == 0 and c["bad_lag"] == 0 and c["bad_smooth"] == 0 else 1)
 
     # configs[0]: the reference's own CPU-runnable case, verbatim run() bodies (mode A)
     N, H, sr = 1024, 512, 44100.0

@@ -1,14 +1,15 @@
-"""Static per-phase SASS instruction count of k_analyse<R1, MG> from the built library (no GPU needed): every instruction is
+"""Static per-phase SASS instruction count of k_analyse<R1, MG, SP> from the built library (no GPU needed): every instruction is
 attributed to the OUTERMOST source line of its inline chain (nvdisasm -gi) and mapped to a phase through the `// ====`
 section markers of fx_analyse.cu, as tools/ncu_phases.py does with executed counts.  Inner loops count once, so this is a
 proxy for the executed instructions per frame -- good for comparing builds before spending GPU time.
-Usage: sass_phases.py [R1=16] [MG=0] [lib]"""
+Usage: sass_phases.py [R1=16] [MG=0] [lib] [SP=0]"""
 import collections, os, re, subprocess, sys, tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 R1 = int(sys.argv[1]) if len(sys.argv) > 1 else 16
 MG = int(sys.argv[2]) if len(sys.argv) > 2 else 0
 lib = sys.argv[3] if len(sys.argv) > 3 else os.path.join(ROOT, "feature-extractor_b200/lib/libfxb200.so")
+SP = int(sys.argv[4]) if len(sys.argv) > 4 else 0
 src = open(os.path.join(ROOT, "feature-extractor_b200/csrc/fx_analyse.cu")).read().split("\n")
 
 
@@ -38,7 +39,7 @@ with tempfile.TemporaryDirectory() as td:
     subprocess.run(["cuobjdump", "-xelf", "all", lib], cwd=td, check=True, stdout=subprocess.DEVNULL)
     cub = [f for f in os.listdir(td) if f.startswith("fx_analyse.") and f.endswith(".cubin")][0]
     sass = subprocess.run(["nvdisasm", "-gi", "-c", os.path.join(td, cub)], capture_output=True, text=True).stdout.split("\n")
-want = f"k_analyseILi{R1}ELb{MG}E"
+want = f"k_analyseILi{R1}ELb{MG}ELb{SP}E"
 inside, cur, counts, core = False, None, collections.Counter(), collections.Counter()
 for l in sass:
     if l.startswith(".text."):
@@ -59,7 +60,7 @@ for l in sass:
         else:
             core[cur[0]] += 1
 tot = sum(counts.values()) + sum(core.values())
-print(f"# static SASS instructions of k_analyse<{R1},{'true' if MG else 'false'}> by phase ({tot} in all; fft_core is a separate function)")
+print(f"# static SASS instructions of k_analyse<{R1},{'true' if MG else 'false'},{'true' if SP else 'false'}> by phase ({tot} in all; fft_core is a separate function)")
 for name, _ in marks[:-1]:
     print(f"{name:40s} {counts[name]:6d}")
 for f, c in core.items():
