@@ -37,79 +37,11 @@
 //     sum (mag / maxE - mean)^2 = S4 / maxE^2 - M mean^2                    (:182-190)
 // in fp64 (the cancellation costs a few of its 16 digits on features compared at 1e-4).  K1b forms them.
 //
-// Build switches.  Each restores the previous form of one optimisation so that it can be A/B-timed on a B200 (tools/exp_build.sh,
-// tools/gpu_ab2.sh; the numbers are in DESIGN.md section 7 and profiles/r02_v2*_ab_*.txt).  Several are per window size: at
-// N = 4096 the kernel sits at its 80-register budget and what trims instructions elsewhere makes ptxas spill there.
-// Dropped after measurement and no longer in the source: a MUFU-approximate flatness eps, packed arithmetic in the split, fp32
+// Every optimisation in this file was A/B-timed on a B200 against the form it replaced (DESIGN.md section 7,
+// profiles/r02_v2*_ab_*.txt); the losing forms are gone.  Three are selected per window size (kPackFilter, kFluxF32Cmp,
+// kLhrRange in k_analyse): at N = 4096 the kernel sits at its 80-register budget and what trims instructions elsewhere makes
+// ptxas spill there.  Dropped after measurement: a MUFU-approximate flatness eps, packed arithmetic in the split, fp32
 // cross-warp sums of rms / magnitude / harmonic sums (spills), a per-warp queue dealing the peaks out one per lane (+1 .. 3 %).
-//   FX_B9_EARLY       the frame's last block barrier stands in front of the peak loop instead of behind it (see there)
-//   FX_ROLE_HIGH      the record stage's parts run on the CTA's last warps (the upper bins: fewer peaks) instead of warps 0 / 1 / 4
-//   FX_PACKED_PASSES  the filter pass (sum of squares, gain, decay, ramp) on packed f32x2 instructions: two samples per
-//                     instruction, IEEE per half, the same values
-//   FX_PACK_LAG       likewise the lag products d^2 s (the same values except the order of a thread's 16-term run sum)
-//   FX_GATHER_GROUPS  FFT-beta's ring gather takes one wrapped base per group of loads that cannot wrap inside (hop >= N / 4)
-//   FX_LAZY_CROSS     the position of a thread's first lag under the threshold is only looked for when its minimum is under it
-//   FX_FLUX_F32CMP    "magnitude rose" decided on |Re| (the magnitudes are exact squares), a predicated add instead of selects
-//   FX_PSUM_SLOT      the norm of P rides in the free eighth slot of pass 1's transposed butterfly
-//   FX_LHR_RANGE      the low-energy sum is the magnitude sum of the threads below the boundary bin; only the one thread that
-//                     straddles it tests bins
-//   FX_PBASE_F32      the lag search's cumulative sum enters a segment as an fp32 sum of the fp32 warp totals (needs FX_PSCAN_F32)
-//   FX_PREFIX_F32     the mantissa of the flatness product's prefix over the preceding warps is fp32 (needs FX_MESCAN_F32)
-#ifndef FX_B9_EARLY
-#define FX_B9_EARLY 1
-#endif
-#ifndef FX_ROLE_HIGH
-#define FX_ROLE_HIGH 1
-#endif
-#ifndef FX_PACKED_PASSES
-#define FX_PACKED_PASSES 2                // 0 never, 1 always, 2 for N <= 2048
-#endif
-#ifndef FX_PACK_LAG
-#define FX_PACK_LAG 1
-#endif
-#ifndef FX_GATHER_GROUPS
-#define FX_GATHER_GROUPS 1
-#endif
-#ifndef FX_LAZY_CROSS
-#define FX_LAZY_CROSS 1
-#endif
-#ifndef FX_FLUX_F32CMP
-#define FX_FLUX_F32CMP 2                  // 0 never, 1 always, 2 for N <= 2048
-#endif
-#ifndef FX_PSUM_SLOT
-#define FX_PSUM_SLOT 1                    // 0 never, 1 always, 2 for N <= 2048 (re-timed on v30: -0.3 % at N = 4096 as well)
-#endif
-#ifndef FX_LHR_RANGE
-#define FX_LHR_RANGE 3                    // 0 never, 1 always, 3 for N >= 2048 (at N = 1024 it costs 0.8 %: spills)
-#endif
-#ifndef FX_PBASE_F32
-#define FX_PBASE_F32 1
-#endif
-#ifndef FX_PREFIX_F32
-#define FX_PREFIX_F32 1
-#endif
-//   FX_LAGSLOT_F32    the lag search's per-warp slot carries the harmonic sum as the fp32 value it is, next to the largest |Re A|: the
-//                     cross-warp sum behind the barrier is an FADD chain and the separate maxima loads go (needs FX_HSUM_F32)
-#ifndef FX_LAGSLOT_F32
-#define FX_LAGSLOT_F32 1
-#endif
-// fp32 warp reductions of sums whose per-thread partials are fp32-accurate anyway (the cross-warp sums stay fp64):
-//   FX_RMS_F32    sum of squares of the frame (16 fp32 squares per thread)
-//   FX_HSUM_F32   harmonic magnitude sum (8 squares per thread)
-//   FX_PSCAN_F32  warp scan of the lag search's cumulative sum (the reference runs this sum in fp32 sequentially, :138-145)
-//   FX_INHARM_F32 inharmonicity sum (a few peaks per thread)                                         (default in fx_kernels.cuh)
-//   FX_P1SUM_F32  pass 1's seven sums (fp64 per thread over its 8 bins, fp32 across the lanes)        (default in fx_kernels.cuh)
-//   FX_MESCAN_F32 mantissa of the flatness product's warp scan (the exponent is an integer; the product only feeds
-//                 pow (., 1 / count))                                                                (default in fx_kernels.cuh)
-#ifndef FX_RMS_F32
-#define FX_RMS_F32 1
-#endif
-#ifndef FX_HSUM_F32
-#define FX_HSUM_F32 1
-#endif
-#ifndef FX_PSCAN_F32
-#define FX_PSCAN_F32 1
-#endif
 
 namespace fx {
 
@@ -242,13 +174,6 @@ __device__ __forceinline__ ME me_mul (ME a, ME b)
     return r;
 }
 
-template <int K> __device__ __forceinline__ void warp_sum (double (&v)[K])
-{
-    #pragma unroll
-    for (int off = 16; off > 0; off >>= 1)
-        #pragma unroll
-        for (int k = 0; k < K; ++k) v[k] += __shfl_xor_sync (0xffffffffu, v[k], off);
-}
 // Sum K (a power of two <= 8) doubles over the warp with a transposed butterfly: each of the first log2 K steps halves the
 // number of values a lane carries (it keeps one half of the pairs and sends the other half to its partner), the remaining
 // steps are plain butterflies on one value: K - 1 + (5 - log2 K) exchanges instead of 5 K.  Afterwards v[0] of every lane
@@ -298,8 +223,6 @@ template <int R1> struct Smem
     static constexpr int N = D::N, M = N / 2, T = D::T, NW = T / 32;
 
     float2   ex[D::EX_LEN];          // FFT exchange buffer; doubles as two fp32 work arrays (skewed, N*17/16 floats each)
-    float2   tw1[FX_TW1_GLOBAL ? 1 : D::TW1_LEN];     // stage-1 twiddle factors (only when they are not read from the global table)
-    float2   tw2[D::TW2_POWERS ? 1 : D::TW2_LEN];   // stage-2 twiddle table (by powers: the compact table lives in the holes of the ring instead)
     // The sample ring and the P / Re A array are SKEWED by one float4 per 32 floats (sk32 below): a thread reads 16 (8)
     // consecutive floats as float4s, i.e. the lanes of a quarter warp are 64 (32) bytes apart and would share two (four) of the
     // eight 16-byte bank groups; with the skew every quarter warp covers all eight.  Runs of 32 consecutive floats that start at
@@ -309,17 +232,16 @@ template <int R1> struct Smem
     // Per-warp partials every thread reads back after a barrier.  What one reader needs of a warp sits in ONE 16-byte slot: a
     // broadcast LDS.128 per warp instead of one load per value (these reads were ~40 of the 230 LDS per thread and frame).
     struct alignas (16) P1Slot  { double s0; float maxre; float psum; };      // pass 1: magnitude sum, largest |Re|, sum of P^2
-    struct alignas (16) ScanSlot { double m; int e; int pad; };               // flatness product scan, warp totals
-    struct alignas (16) LagSlot { double hsum; unsigned first_cross; unsigned best; };   // harmonic magnitude sum; first lag under the threshold, smallest cnd (bit pattern)
+    struct alignas (16) ScanSlot { double m; int e; float mf; };              // flatness product scan, warp totals (the prefix reads e and mf = (float) m)
+    struct alignas (16) LagSlot { float hsum, hmax; unsigned first_cross, best; };      // harmonic magnitude sum, largest |Re A|; first lag under the threshold, smallest cnd (bit pattern)
     alignas (16) double rms[NW];     // sum of squares of the frame, warp totals
     P1Slot   p1s[NW];
     ScanSlot scan[NW];
-    alignas (16) double pscan[NW];   // pitch cumulative sum scan, warp totals
+    alignas (16) float pscan[NW];    // pitch cumulative sum scan, warp totals
     LagSlot  lags[NW];
-    alignas (16) float hmaxs[NW];    // largest |Re A|, warp maxima
     unsigned ugidx[NW];             // first index holding the smallest cnd (only formed when no lag crosses the threshold)
     unsigned ucodes[NW];            // flatness product: earliest range-event thread of the warp
-    float    fmins[3][NW];           // [0] flatness gate margin, [2] peak margin (diagnostics)
+    float    fmins[2][NW];           // [0] flatness gate margin, [1] peak margin (diagnostics)
     float    pmins[2][NW];           // pitch margin / runner-up partials
     union
     {
@@ -348,18 +270,11 @@ __device__ __noinline__ void fft_core (V16 io, int m0)
 {
     Smem<R1>& sm = *reinterpret_cast<Smem<R1>*> (fx_smem_raw);
     const int t = threadIdx.x;
-    fft_stage1_store<R1, false> (io.v, m0, sm.ex, sm.tw1, sm.tw1f);
-#if FX_STAGE23_SHFL
-    static_assert (! FftDims<R1>::TW2_POWERS, "the experiment paths read the full stage-2 table: build them with -DFX_TW2_POWERS=0");
-#endif
+    fft_stage1_store<R1, false> (io.v, m0, sm.ex, sm.tw1f);
     __syncthreads();
-#if FX_STAGE23_SHFL
-    fft_stage23_shfl<R1, false> (t, sm.ex, sm.tw2);         // experiment: the 2 -> 3 exchange by warp shuffles (measured slower)
-#else
-    fft_stage2<R1, false> (t, sm.ex, FftDims<R1>::TW2_POWERS ? reinterpret_cast<const float2*> (sm.ring + 32) : sm.tw2);
+    fft_stage2<R1, false, true> (t, sm.ex, reinterpret_cast<const float2*> (sm.ring + 32));
     __syncwarp();                                           // rows are private to a half warp from here on
     fft_stage3<R1, false> (t, sm.ex);
-#endif
 }
 
 // MG: also compute the decision margins (diagnostics, FX_DIAG_*_MARGIN).  They feed nothing: a call that does not ask for the
@@ -369,42 +284,40 @@ __device__ __noinline__ void fft_core (V16 io, int m0)
 // (N = 2048 / 1024: 28 / 26 warps per SM instead of 24; the seventh / thirteenth CTA fits the shared memory only with the compact
 // stage-2 twiddle table, 512 B instead of 1920 B).  Measured against 6 / 12 CTAs at 80 registers: 32.45 vs 32.78 ms at N = 2048,
 // 33.82 vs 33.98 ms at N = 1024 (profiles/r02_v23_ab_occupancy.txt).
-#ifndef FX_CTAS_R8
-#define FX_CTAS_R8 7
-#endif
-#ifndef FX_CTAS_R4
-#define FX_CTAS_R4 13
-#endif
+constexpr int kCtasR16 = 3, kCtasR8 = 7, kCtasR4 = 13;
 // (233 472 bytes of shared memory per SM, 1 KB of it reserved per resident CTA)
-static_assert (3 * (sizeof (Smem<16>) + 1024) <= 233472, "three CTAs of N = 4096 per SM");
-static_assert (FX_CTAS_R8 * (sizeof (Smem<8>) + 1024) <= 233472, "resident CTAs of N = 2048 per SM");
-static_assert (FX_CTAS_R4 * (sizeof (Smem<4>) + 1024) <= 233472, "resident CTAs of N = 1024 per SM");
+static_assert (kCtasR16 * (sizeof (Smem<16>) + 1024) <= 233472, "three CTAs of N = 4096 per SM");
+static_assert (kCtasR8 * (sizeof (Smem<8>) + 1024) <= 233472, "resident CTAs of N = 2048 per SM");
+static_assert (kCtasR4 * (sizeof (Smem<4>) + 1024) <= 233472, "resident CTAs of N = 1024 per SM");
 // SP: power-spectrum mode (FX_SPECTRUM_POWER).  Each of the three spectra is handed on as (|X[k]|, 0) instead of
 // (Re X[k], Im X[k]): |B| to the spectral passes and the previous spectrum, P = |C|^2 to FFT-beta, |A| to the harmonic
 // pass.  Everything downstream squares or compares these values exactly as it squares and compares Re, so the two
 // places that form them (the split after FFT-alpha, the hand-over of A after FFT-beta) are the only branches on SP;
 // the instantiations without it are the parity mode, unchanged.
 template <int R1, bool MG, bool SP>
-__global__ void __launch_bounds__ (16 * R1, (R1 == 16 ? 3 : (R1 == 8 ? FX_CTAS_R8 : FX_CTAS_R4)))
+__global__ void __launch_bounds__ (16 * R1, (R1 == 16 ? kCtasR16 : (R1 == 8 ? kCtasR8 : kCtasR4)))
 k_analyse (const AnalyseParams p)
 {
     using D = FftDims<R1>;
     using S = Smem<R1>;
     constexpr int N = D::N, M = N / 2, T = D::T, NW = T / 32, Q1 = D::Q1;
     constexpr int LOG_N = R1 == 16 ? 12 : (R1 == 8 ? 11 : 10);
-    // measured per size (profiles/r02_v28_ab_*.txt): the packed filter pass and the |Re| flux test pay 1.2 - 2.1 % at N = 2048 / 1024
-    // (no spills there) and cost 2.7 % at N = 4096 (80-register budget: 40 bytes of spills)
-    // (which of the three takes which part is immaterial: profiles/r02_v29c_ab_role_permutations_4096.txt)
-    constexpr int kRoleHer  = FX_ROLE_HIGH ? NW - 1 : 0;
-    constexpr int kRoleHead = FX_ROLE_HIGH ? (NW >= 2 ? NW - 2 : 0) : 1 % NW;
-    constexpr int kRoleFlat = FX_ROLE_HIGH ? (NW >= 3 ? NW - 3 : 0) : 4 % NW;
-    constexpr bool kPackFilter = FX_PACKED_PASSES == 1 || (FX_PACKED_PASSES == 2 && R1 <= 8);
-    // (its three parts -- sums of squares, the (x gain, x c1 gain) multiply, decay + ramp -- were also timed alone at N = 4096:
-    // 0 / +0.1 / +2.1 %, profiles/r02_v29a_ab_4096.txt)
-    constexpr bool kPackSq = kPackFilter, kPackXg = kPackFilter, kPackTail = kPackFilter;
-    constexpr bool kFluxF32Cmp = FX_FLUX_F32CMP == 1 || (FX_FLUX_F32CMP == 2 && R1 <= 8);
-    constexpr bool kPsumSlot = FX_PSUM_SLOT == 1 || (FX_PSUM_SLOT == 2 && R1 <= 8);
-    constexpr bool kLhrRange = FX_LHR_RANGE == 1 || (FX_LHR_RANGE == 3 && R1 >= 8);
+    // The record stage's parts run on the CTA's last warps: the upper bins have fewer peaks, so those warps leave the peak
+    // loop first (which of the three takes which part is immaterial: profiles/r02_v29c_ab_role_permutations_4096.txt)
+    constexpr int kRoleHer  = NW - 1;
+    constexpr int kRoleHead = NW >= 2 ? NW - 2 : 0;
+    constexpr int kRoleFlat = NW >= 3 ? NW - 3 : 0;
+    // Per window size (profiles/r02_v28a_ab_*.txt): the filter pass on packed f32x2 instructions (two samples per instruction,
+    // IEEE per half: the same values) pays 1.2 - 1.4 % at N = 2048 / 1024 (no spills there) and costs 2.7 % at N = 4096
+    // (80-register budget: 40 bytes of spills).  Its three parts -- sums of squares, the (x gain, x c1 gain) multiply, decay +
+    // ramp -- were also timed alone at N = 4096: 0 / +0.1 / +2.1 % (profiles/r02_v29a_ab_4096.txt).
+    constexpr bool kPackFilter = R1 <= 8;
+    // Per window size (profiles/r02_v26a_ab_*.txt, r02_v28a_ab_*.txt): "magnitude rose" decided on |Re| with a predicated add
+    // instead of selects on the fp64 difference trims instructions where they fit and spills at N = 4096 (+0.6 % there).
+    constexpr bool kFluxF32Cmp = R1 <= 8;
+    // Per window size (profiles/r02_v28b_ab_*.txt): the low-energy sum as the magnitude sum of the threads below the boundary
+    // bin, only the thread that straddles it testing bins, pays at N >= 2048 and costs 0.8 % at N = 1024 (spills).
+    constexpr bool kLhrRange = R1 >= 8;
 
     S& sm = *reinterpret_cast<S*> (fx_smem_raw);
     float* workf = reinterpret_cast<float*> (sm.ex);          // fp32 view, skewed index phys (n)
@@ -427,14 +340,11 @@ k_analyse (const AnalyseParams p)
     const float* src = p.audio + track * p.track_stride;
     const float* tail = p.tail_in + track * (long) (N - H);
 
-    if (! FX_TW1_GLOBAL) for (int i = t; i < D::TW1_LEN; i += T) sm.tw1[i] = p.tw1[i];
-    if (D::TW2_POWERS)                                                                            // rows k2 = 1, 2, 4, 8, into the ring's holes
-    {
-        static_assert (D::TW2_LEN / 2 <= N / 32, "one hole per two stage-2 twiddles");
-        for (int i = t; i < D::TW2_LEN; i += T)
-            reinterpret_cast<float2*> (sm.ring + 32)[18 * (i >> 1) + (i & 1)] = p.tw2[((1 << (i >> 4)) - 1) * 16 + (i & 15)];
-    }
-    else               { for (int i = t; i < D::TW2_LEN; i += T) sm.tw2[i] = p.tw2[i]; }
+    // The stage-2 twiddles by powers (fx_fft.cuh), rows k2 = 1, 2, 4, 8, live in the ring's holes.  At N = 2048 / 1024 they
+    // cost ~1 % by themselves and buy the shared memory for one more resident CTA: 512 B instead of the full table's 1920 B.
+    static_assert (4 * 16 / 2 <= N / 32, "one hole per two stage-2 twiddles");
+    for (int i = t; i < 4 * 16; i += T)
+        reinterpret_cast<float2*> (sm.ring + 32)[18 * (i >> 1) + (i & 1)] = p.tw2[((1 << (i >> 4)) - 1) * 16 + (i & 15)];
     if (t == 0) { mbar_init (&sm.mbar, T); sm.tw1f = p.tw1f; }             // every thread arrives once per hop block (its copies, or its stores)
     asm volatile ("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
@@ -511,7 +421,7 @@ k_analyse (const AnalyseParams p)
             {
                 const float4 x4 = *reinterpret_cast<const float4*> (&sm.ring[r0 + 4 * q]);
                 xs[4 * q] = x4.x; xs[4 * q + 1] = x4.y; xs[4 * q + 2] = x4.z; xs[4 * q + 3] = x4.w;
-                if (kPackSq)
+                if (kPackFilter)
                 {
                     sqp = f2fma (make_float2 (x4.x, x4.y), make_float2 (x4.x, x4.y), sqp); sqp = f2fma (make_float2 (x4.z, x4.w), make_float2 (x4.z, x4.w), sqp);
                 }
@@ -520,21 +430,15 @@ k_analyse (const AnalyseParams p)
                     sq0 = fmaf (x4.x, x4.x, sq0); sq1 = fmaf (x4.y, x4.y, sq1); sq0 = fmaf (x4.z, x4.z, sq0); sq1 = fmaf (x4.w, x4.w, sq1);
                 }
             }
-            if (kPackSq)
+            if (kPackFilter)
             {
                 sq0 = sqp.x; sq1 = sqp.y;
             }
             {
-#if FX_RMS_F32
                 const float wsq = warp_sumf (sq0 + sq1);
                 if (lane == 0) sm.rms[warp] = (double) wsq * ((double) gain * (double) gain);      // AudioDataCollector.h:88 applies the gain
-#else
-                double r1[1] = { (double) (sq0 + sq1) * ((double) gain * (double) gain) };       // AudioDataCollector.h:88 applies the gain
-                warp_sum<1> (r1);
-                if (lane == 0) sm.rms[warp] = r1[0];
-#endif
             }
-            if (kPackXg)
+            if (kPackFilter)
             {
                 // (x gain, x c1 gain) of a sample in one packed multiply: the first half is the windowed path's sample, the second the filter's input
                 #pragma unroll
@@ -576,7 +480,7 @@ k_analyse (const AnalyseParams p)
                                            3.132781128e-08f, 6.512412136e-09f };
             // Both windowed sequences go to the exchange buffer in natural (skewed) order as the packed input of FFT-alpha,
             // z[n] = x[n] w[n] + i y[n] w[n]: the transform's strided gather is then one 8-byte load per point.
-            if (kPackTail)
+            if (kPackFilter)
             {
                 // (two samples per instruction: the neighbour's decaying contribution, the ramp, and each sample's two sequences by its ramp value)
                 #pragma unroll
@@ -589,8 +493,8 @@ k_analyse (const AnalyseParams p)
                     // (what is stored is z / 2 -- see the split below)
                     const float2 w2 = f2fma (make_float2 ((float) j, (float) (j + 1)), make_float2 (wseg_d, wseg_d), make_float2 (wseg_0, wseg_0));
                     float2* zp = &sm.ex[(t >> 4) * D::ROW + 17 * (t & 15) + j];                                                   // tpos (16 t + j)
-                    zp[0] = f2mul (make_float2 (kPackXg ? xg[j] : __fmul_rn (xs[j], gain), y2.x), make_float2 (w2.x, w2.x));
-                    zp[1] = f2mul (make_float2 (kPackXg ? xg[j + 1] : __fmul_rn (xs[j + 1], gain), y2.y), make_float2 (w2.y, w2.y));
+                    zp[0] = f2mul (make_float2 (xg[j], y2.x), make_float2 (w2.x, w2.x));
+                    zp[1] = f2mul (make_float2 (xg[j + 1], y2.y), make_float2 (w2.y, w2.y));
                 }
             }
             else
@@ -740,21 +644,17 @@ k_analyse (const AnalyseParams p)
                 }
             }
             lprod = me_from (mprod); lprod.e += esum;
-#if FX_P1SUM_F32
-            float s8[8] = { (float) mag_sum, (float) weighted, (float) flux, (float) lhr, (float) s2, (float) s4, (float) flat_sum, kPsumSlot ? psum : 0.0f };
-#else
-            double s8[8] = { mag_sum, weighted, flux, lhr, s2, s4, flat_sum, kPsumSlot ? (double) psum : 0.0 };
-#endif
+            // the norm of P rides in the free eighth slot of the transposed butterfly (profiles/r02_v31_ab_psum_always_4096.txt)
+            float s8[8] = { (float) mag_sum, (float) weighted, (float) flux, (float) lhr, (float) s2, (float) s4, (float) flat_sum, psum };
             warp_sum_t<8> (s8, lane);
             const int wcount = warp_addi (count);
             const float wmax = warp_max_nonneg (maxre);
             const float wraw = warp_max_nonneg (rawmax);
-            const float wps = kPsumSlot ? (float) __shfl_sync (0xffffffffu, s8[0], 7)              // slot 7's total lives in lanes = 7 mod 8
-                                        : warp_sumf (psum);
+            const float wps = __shfl_sync (0xffffffffu, s8[0], 7);                                  // slot 7's total lives in lanes = 7 mod 8
             float wmar = 1.0f;
             if (MG) wmar = warp_min_nonneg (fminf (gate_d * gate_inv, 0.5f));
-            // inclusive warp scan of the extended-range product, in bin order
-#if FX_MESCAN_F32
+            // inclusive warp scan of the extended-range product, in bin order; the mantissa in fp32 (the exponent is an integer,
+            // and the product only feeds pow (., 1 / count))
             struct { float m; int e; } incf = { (float) lprod.m, lprod.e };                      // m in [0.5, 1]
             #pragma unroll
             for (int off = 1; off < 32; off <<= 1)
@@ -768,15 +668,6 @@ k_analyse (const AnalyseParams p)
                 }
             }
             ME inc; inc.m = (double) incf.m; inc.e = incf.e;
-#else
-            ME inc = lprod;
-            #pragma unroll
-            for (int off = 1; off < 32; off <<= 1)
-            {
-                ME o; o.m = __shfl_up_sync (0xffffffffu, inc.m, off); o.e = __shfl_up_sync (0xffffffffu, inc.e, off);
-                if (lane >= off) inc = me_mul (o, inc);
-            }
-#endif
             ME exc; exc.m = __shfl_up_sync (0xffffffffu, inc.m, 1); exc.e = __shfl_up_sync (0xffffffffu, inc.e, 1);
             if (lane == 0) exc = me_one();
             lprod = exc;                                                                         // lane-exclusive prefix within the warp
@@ -803,7 +694,7 @@ k_analyse (const AnalyseParams p)
         double mag_sum_acc = 0.0;
         float maxre_all = 0.0f, psum_all = 0.0f;
         ME prefix = me_one();
-        float pfm = 0.5f; int pfe = 1; (void) pfm; (void) pfe;
+        float pfm = 0.5f; int pfe = 1;
         // every thread needs the magnitude sum (silence gate), the largest |Re| (exponent budget below) and the norm of P;
         // everything else of the pass has already left for K1b as per-warp partials
         #pragma unroll
@@ -819,17 +710,11 @@ k_analyse (const AnalyseParams p)
         for (int w = 0; w < warp; ++w)
         {
             const double2 sl = *reinterpret_cast<const double2*> (&sm.scan[w]);
-#if FX_PREFIX_F32 && FX_MESCAN_F32
             const float wm = __int_as_float (__double2hiint (sl.y));                              // the warp total's fp32 mantissa rides in the slot's spare word
             pfm *= wm; pfe += __double2loint (sl.y);
             if (pfm < 0.5f) { pfm *= 2.0f; pfe -= 1; }
-#else
-            ME wt; wt.m = sl.x; wt.e = __double2loint (sl.y); prefix = me_mul (prefix, wt);
-#endif
         }
-#if FX_PREFIX_F32 && FX_MESCAN_F32
         prefix.m = (double) pfm; prefix.e = pfe;
-#endif
         prefix = me_mul (prefix, lprod);
         const double maxmag = (double) maxre_all * (double) maxre_all;
         const bool silent = ! (mag_sum > 0.05);                                                   // :121-123
@@ -915,7 +800,7 @@ k_analyse (const AnalyseParams p)
             const int rg = (int) ((a0 + t) >> 5) & (N / 32 - 1), rl = (int) ((a0 + t) & 31);
             const int pa_up = 36 * warp + lane;                                                   // sk32 (c + t) - 36 (c / 32)
             const int pa_dn = -36 * warp - lane - (lane ? 4 : 0);                                 // sk32 (N - c - t) - 36 ((N - c) / 32)
-            if (FX_GATHER_GROUPS && NB <= 4)
+            if (NB <= 4)
             {
                 // the window starts at a multiple of the hop: with hop >= N / 4 the ring wraps at a multiple of N / 4 samples, never
                 // inside a quarter of the window -- one wrapped base per quarter, compile-time offsets inside it
@@ -986,7 +871,7 @@ k_analyse (const AnalyseParams p)
         {
             const float s0f = (float) (16 * t);
             float runf = 0.0f;
-#if FX_PACK_LAG
+            // two lags per packed instruction: the same values except the order of a thread's 16-term run sum
             float2 run2 = make_float2 (0.0f, 0.0f);
             #pragma unroll
             for (int j = 0; j < 16; j += 2)
@@ -1002,16 +887,6 @@ k_analyse (const AnalyseParams p)
                 run2 = f2add (run2, a2);
             }
             runf = run2.x + run2.y;
-#else
-            #pragma unroll
-            for (int j = 0; j < 16; ++j)
-            {
-                const float d = sm.ex[zl_own + zrun<R1> (j)].y + sm.ex[j == 0 ? zl_self : zl_mirror + zrun<R1> (16 - j)].y;     // Z[s] + Z[N - s]: 2 * 2^k * D[s]
-                if (MG) dv[j] = d;
-                av[j] = __fmul_rn (__fmul_rn (d, d), __fadd_rn (s0f, (float) j));                 // s = 0 contributes 0 (one FADD: the sum is exact)
-                runf += av[j];
-            }
-#endif
             // Re A of this thread's 8 bins moves to the P / Re A array (P was consumed by the transform).  Power mode: |A|, with
             // Im A[k] = (Im Z[k] - Im Z[N-k]) / 2 -- Im A is odd and 2^k D even, so D cancels.
             {
@@ -1030,7 +905,7 @@ k_analyse (const AnalyseParams p)
                 *reinterpret_cast<float4*> (&sm.pa[pb0])     = make_float4 (ra[0], ra[1], ra[2], ra[3]);
                 *reinterpret_cast<float4*> (&sm.pa[pb0 + 4]) = make_float4 (ra[4], ra[5], ra[6], ra[7]);
             }
-#if FX_PSCAN_F32
+            // warp scan of the cumulative sum in fp32 (the reference runs this sum in fp32 sequentially, :138-145)
             float inc = runf;
             #pragma unroll
             for (int off = 1; off < 32; off <<= 1)
@@ -1040,50 +915,22 @@ k_analyse (const AnalyseParams p)
             }
             const float excf = __shfl_up_sync (0xffffffffu, inc, 1);
             seg_exc = lane == 0 ? 0.0 : (double) excf;
-#if FX_PBASE_F32
-            if (lane == 31) reinterpret_cast<float*> (sm.pscan)[warp] = inc;
-#else
-            if (lane == 31) sm.pscan[warp] = (double) inc;
-#endif
-#else
-            double inc = (double) runf;
-            #pragma unroll
-            for (int off = 1; off < 32; off <<= 1)
-            {
-                const double o = __shfl_up_sync (0xffffffffu, inc, off);
-                if (lane >= off) inc += o;
-            }
-            seg_exc = __shfl_up_sync (0xffffffffu, inc, 1);
-            if (lane == 0) seg_exc = 0.0;
             if (lane == 31) sm.pscan[warp] = inc;
-#endif
             if (MG && t == 0) sm.d0 = dv[0];
         }
         __syncthreads();
         unsigned first_cross = 0xffffffffu, nd_mask = 0u, wfc, wbest;
         {
-#if FX_PBASE_F32 && FX_PSCAN_F32
+            // the segment's running sum starts from the fp32 sum of the preceding warps' fp32 totals
             float sumf = 0.0f;
             #pragma unroll
             for (int w = 0; w < NW; w += 2)
             {
-                const float2 p2 = *reinterpret_cast<const float2*> (&reinterpret_cast<const float*> (sm.pscan)[w]);
+                const float2 p2 = *reinterpret_cast<const float2*> (&sm.pscan[w]);
                 if (w < warp) sumf += p2.x;
                 if (w + 1 < warp) sumf += p2.y;
             }
             sumf += (float) seg_exc;
-#else
-            double base = seg_exc;
-            #pragma unroll
-            for (int w = 0; w < NW; w += 2)
-            {
-                const double2 p2 = *reinterpret_cast<const double2*> (&sm.pscan[w]);
-                if (w < warp) base += p2.x;
-                if (w + 1 < warp) base += p2.y;
-            }
-            // fp32 running sum inside the segment, as in the reference (:138-145), on top of the fp64 prefix
-            float sumf = (float) base;
-#endif
             float best = 100.0f;
             unsigned cross = 0u;
             float c_before = 0.0f;
@@ -1099,13 +946,9 @@ k_analyse (const AnalyseParams p)
                 c_before = c;
                 if (j >= 2 || t != 0)                                                             // the search starts at s = 2 (:169)
                 {
-#if ! FX_LAZY_CROSS
-                    if (c < 0.01f) cross |= 1u << j;                                              // :176
-#endif
                     best = fminf (best, c);                                                       // :171-175 (its index only matters when no lag crosses: found then)
                 }
             }
-#if FX_LAZY_CROSS
             // :176 some lag of this thread is under the threshold iff its minimum is: only then (few threads of a frame) look for the first
             if (best < 0.01f)
             {
@@ -1113,7 +956,6 @@ k_analyse (const AnalyseParams p)
                 for (int j = 15; j >= 0; --j)
                     if ((j >= 2 || t != 0) && workg[17 * t + j] < 0.01f) cross = 1u << j;        // (this thread's own stores)
             }
-#endif
             sm.ndm[t] = (unsigned short) nd_mask;
             if (cross != 0u) first_cross = (unsigned) (16 * t + __ffs ((int) cross) - 1);
             // smallest cnd of the warp (cnd >= 0 orders like its bit pattern)
@@ -1132,35 +974,18 @@ k_analyse (const AnalyseParams p)
             ar[1] = (b0 >= 1) ? sm.pa[sk32 (b0 - 2) + 1] : 0.0f;
             ar[10] = (b0 + 8 < M) ? sm.pa[sk32 (b0 + 8)] : 0.0f;
             float hmaxre = 0.0f;
-#if FX_HSUM_F32
             float hsf = 0.0f;
             #pragma unroll
             for (int j = 0; j < 8; ++j) { hsf = fmaf (ar[2 + j], ar[2 + j], hsf); hmaxre = fmaxf (hmaxre, fabsf (ar[2 + j])); }
             double s1[1] = { (double) warp_sumf (hsf) };
-#else
-            double hsum = 0.0;
-            #pragma unroll
-            for (int j = 0; j < 8; ++j) { const double re = (double) ar[2 + j]; hsum += re * re; hmaxre = fmaxf (hmaxre, fabsf (ar[2 + j])); }
-            double s1[1] = { hsum };
-            warp_sum<1> (s1);
-#endif
             const float wm = warp_max_nonneg (hmaxre);
-            if (lane == 0)
-            {
-#if FX_LAGSLOT_F32 && FX_HSUM_F32
-                *reinterpret_cast<float4*> (&sm.lags[warp]) = make_float4 ((float) s1[0], wm, __uint_as_float (wfc), __uint_as_float (wbest));
-#else
-                *reinterpret_cast<double2*> (&sm.lags[warp]) = make_double2 (s1[0], __hiloint2double ((int) wbest, (int) wfc));
-                sm.hmaxs[warp] = wm;
-#endif
-            }
+            if (lane == 0) *reinterpret_cast<float4*> (&sm.lags[warp]) = make_float4 ((float) s1[0], wm, __uint_as_float (wfc), __uint_as_float (wbest));
         }
         __syncthreads();
         // ---- every thread now derives the lag on its own (all control flow below is uniform across the CTA) -----------
         unsigned s0 = 0xffffffffu;
         unsigned gbest = 0xffffffffu;                              // bit pattern of the smallest cnd of the search range
         float hmaxre = 0.0f;
-#if FX_LAGSLOT_F32 && FX_HSUM_F32
         float hsum_acc = 0.0f;
         #pragma unroll
         for (int w = 0; w < NW; ++w)
@@ -1171,33 +996,7 @@ k_analyse (const AnalyseParams p)
             hsum_acc += sl.x;
             hmaxre = fmaxf (hmaxre, sl.y);
         }
-#else
-        double hsum_acc = 0.0;
-        #pragma unroll
-        for (int w = 0; w < NW; ++w)
-        {
-            const double2 sl = *reinterpret_cast<const double2*> (&sm.lags[w]);                   // one LDS.128: { hsum, (first_cross, best) }
-            s0 = min (s0, (unsigned) __double2loint (sl.y));
-            gbest = min (gbest, (unsigned) __double2hiint (sl.y));
-            hsum_acc += sl.x;
-        }
-#endif
         const double hsum = (double) hsum_acc;
-        if (FX_LAGSLOT_F32 && FX_HSUM_F32) { }
-        else if (NW >= 4)
-        {
-            #pragma unroll
-            for (int w = 0; w + 3 < NW; w += 4)
-            {
-                const float4 h4 = *reinterpret_cast<const float4*> (&sm.hmaxs[w]);
-                hmaxre = fmaxf (fmaxf (hmaxre, fmaxf (h4.x, h4.y)), fmaxf (h4.z, h4.w));
-            }
-        }
-        else
-        {
-            const float2 h2 = *reinterpret_cast<const float2*> (&sm.hmaxs[0]);
-            hmaxre = fmaxf (h2.x, h2.y);
-        }
         const double hmax = (double) hmaxre * (double) hmaxre;
         const bool crossed = (s0 != 0xffffffffu);
         const float e_abs = MG ? 1.0e-6f * fabsf (sm.d0) : 0.0f;
@@ -1280,14 +1079,12 @@ k_analyse (const AnalyseParams p)
             const float wpm = warp_min_nonneg (pm);
             if (lane == 0) sm.pmins[0][warp] = wpm;
         }
-#if FX_B9_EARLY
         // The frame's last block barrier: every read of the cnd values (the exchange buffer, which the next frame's filter pass
         // overwrites) and of the descent masks (whose storage the record stage reuses) is behind it.  The peak loop below -- a
         // thread-dependent number of peaks -- and the record stage then run into the next frame's filter pass without another
         // barrier: their imbalance is absorbed once, at the barrier behind that pass, not twice.  What they read (this thread's
         // registers, the P / Re A array, per-warp slots of earlier phases) is not written again before the next frame's pass 1.
         __syncthreads();
-#endif
         // The harmonic and sub-octave bins of f0 = sample rate / lag come from a table built on the host with the reference's
         // own double arithmetic (PitchAnalyser.h:57, HarmonicCharacteristics.h:158-185): slot 0 stands for lag -1
         const int lag_slot = lag_i < 0 ? 0 : lag_i;
@@ -1396,17 +1193,12 @@ k_analyse (const AnalyseParams p)
             const float pkm = ulps_to_margin (pgap);
             // (the normalised magnitudes of :71-77 are not materialised: their sum is magnitudeSum / maxMagnitude up to fp64
             // rounding, and the few the harmonic energy terms look at are formed from Re A by the record stage)
-#if FX_INHARM_F32
             double s1[1] = { (double) warp_sumf ((float) inharm) };
-#else
-            double s1[1] = { inharm };
-            warp_sum<1> (s1);
-#endif
             const int wnp = warp_addi (npeaks);
             if (lane == 0) { rec_w[warp].inharm = s1[0]; rec_w[warp].npeaks = wnp; }           // K1b sums the warps' parts
-            if (MG) { const float wpk = warp_min_nonneg (pkm); if (lane == 0) sm.fmins[2][warp] = wpk; }
+            if (MG) { const float wpk = warp_min_nonneg (pkm); if (lane == 0) sm.fmins[1][warp] = wpk; }
         }
-        if (MG || ! FX_B9_EARLY) __syncthreads();                     // (the margins' per-warp minima reach the warp that records them)
+        if (MG) __syncthreads();                     // (the margins' per-warp minima reach the warp that records them)
         // ---- what is left of the frame's record ----------------------------------------------------------------------
         // The sums only K1b looks at left as per-warp partials where they were formed (the record's WarpParts); what remains here are the
         // values every thread holds (lag, harmonic sum and maximum), the 18 harmonic-energy maxima, the margins (MG) and the
@@ -1439,7 +1231,7 @@ k_analyse (const AnalyseParams p)
                 float pkm = 1.0f, pmm = 1.0f;
                 if (MG)
                 {
-                    pkm = warp_min_nonneg (ld ? sm.fmins[2][lane] : 1.0f);
+                    pkm = warp_min_nonneg (ld ? sm.fmins[1][lane] : 1.0f);
                     pmm = warp_min_nonneg (ld ? sm.pmins[0][lane] : 1.0f);
                     const float second = warp_min_nonneg (ld ? sm.pmins[1][lane] : 100.0f);
                     if (! crossed) pmm = fminf (pmm, relmargin_f (__uint_as_float (gbest), second));
@@ -1521,16 +1313,10 @@ k_analyse (const AnalyseParams p)
 // the staged records would cap them: a block of 12 warps therefore shares THREE staging buffers in turn.  Warp w waits for
 // its batch in buffer w % 3, reduces the per-warp partials of its 32 frames into registers, hands the buffer to batch
 // w + 3 (it issues that copy itself: no "buffer empty" barrier) and runs the tail while the later batches stream in.
-#ifndef FX_FZ_WARPS
-#define FX_FZ_WARPS 12
-#endif
-#ifndef FX_FZ_BLOCKS
-#define FX_FZ_BLOCKS 2
-#endif
-constexpr int kFzWarps = FX_FZ_WARPS, kFzBufs = 3;
+constexpr int kFzWarps = 12, kFzBufs = 3, kFzBlocks = 2;
 constexpr int kFinalizeRows = 32 * kFzWarps;
 template <int NW>
-__global__ void __launch_bounds__ (kFinalizeRows, FX_FZ_BLOCKS) k_finalize (const FinalizeParams p)
+__global__ void __launch_bounds__ (kFinalizeRows, kFzBlocks) k_finalize (const FinalizeParams p)
 {
     constexpr size_t RB = sizeof (FrameHead) + NW * sizeof (WarpPart);
     constexpr size_t BB = 32 * RB;
@@ -1747,7 +1533,7 @@ template <int R1> static cudaError_t configure_t()
 
 int analyse_ctas_per_sm (int window)
 {
-    return window == 4096 ? 3 : (window == 2048 ? FX_CTAS_R8 : FX_CTAS_R4);
+    return window == 4096 ? kCtasR16 : (window == 2048 ? kCtasR8 : kCtasR4);
 }
 
 size_t analyse_smem_bytes (int window)

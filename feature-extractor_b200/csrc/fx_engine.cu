@@ -80,7 +80,7 @@ struct fx_engine
     std::mutex api_mutex;                // offline calls, parameter calls, fx_process, start / stop
     std::atomic<uint64_t> launches{0};
 
-    float2 *d_tw1 = nullptr, *d_tw2 = nullptr, *d_tw1f = nullptr;
+    float2 *d_tw2 = nullptr, *d_tw1f = nullptr;
     double *d_ex_tab = nullptr;
     int    *d_ex_off = nullptr;
     short  *d_her_tab = nullptr;
@@ -233,7 +233,6 @@ fx_status ensure_records (fx_engine* e, long frames)
 int choose_chunks (const fx_engine* e, long n_tracks, long frames)
 {
     if (frames <= 8 || n_tracks <= 0) return 1;
-    if (const char* f = getenv ("FXB200_CHUNKS")) { const long k = atol (f); if (k >= 1 && k <= (frames + 7) / 8) return (int) k; }   // tuning aid
     const long slots = (long) e->sm_count * e->ctas_per_sm;
     const long target = slots * 6;
     const long max_c = (frames + 7) / 8;
@@ -274,7 +273,7 @@ fx_status run_range (fx_engine* e, int t0, int nt, int n_chunks, int flip, long 
     a.want_margins = d_diag != nullptr ? 1 : 0;
     a.gain = e->d_gain + t0;
     a.sample_rate = e->cfg.sample_rate; a.bin_var = e->bin_var; a.iir_c1 = e->iir_c1; a.iir_c2 = e->iir_c2;
-    a.tw1 = e->d_tw1; a.tw2 = e->d_tw2; a.tw1f = e->d_tw1f;
+    a.tw2 = e->d_tw2; a.tw1f = e->d_tw1f;
     a.her_tab = e->d_her_tab; a.ex_tab = e->d_ex_tab; a.ex_off = e->d_ex_off;
     for (int k = 0; k < 16; ++k) a.f0bin_pow2[k] = e->f0bin_pow2[k];
     a.rec = sc.rec;
@@ -347,7 +346,7 @@ void free_engine (fx_engine* e)
     rt_stop_workers (e);
     cudaSetDevice (e->cfg.device);
     cudaDeviceSynchronize();
-    cudaFree (e->d_tw1); cudaFree (e->d_tw2); cudaFree (e->d_tw1f); cudaFree (e->d_her_tab); cudaFree (e->d_ex_tab); cudaFree (e->d_ex_off);
+    cudaFree (e->d_tw2); cudaFree (e->d_tw1f); cudaFree (e->d_her_tab); cudaFree (e->d_ex_tab); cudaFree (e->d_ex_off);
     cudaFree (e->d_gain); cudaFree (e->d_mult); cudaFree (e->d_ratio); cudaFree (e->d_type); cudaFree (e->d_hist); cudaFree (e->d_reset); cudaFree (e->d_start);
     for (int i = 0; i < 2; ++i) { cudaFree (e->d_tail[i]); cudaFree (e->d_prev[i]); cudaFree (e->d_hrows[i]); }
     cudaFree (e->scratch.first_spec); cudaFree (e->scratch.last_spec); cudaFree (e->scratch.first_idx); cudaFree (e->scratch.rec);
@@ -641,11 +640,9 @@ fx_status fx_engine_create (const fx_config* cfg, fx_engine** out)
     FX_CREATE (cudaStreamCreateWithFlags (&e->stream, cudaStreamNonBlocking));
     FX_CREATE (cudaEventCreateWithFlags (&e->ev_last, cudaEventDisableTiming));
 
-    std::vector<float2> tw1, tw2, tw1f;
-    build_twiddles (N, tw1, tw2, tw1f);
-    FX_CREATE (cudaMalloc (&e->d_tw1, tw1.size() * sizeof (float2)));
+    std::vector<float2> tw2, tw1f;
+    build_twiddles (N, tw2, tw1f);
     FX_CREATE (cudaMalloc (&e->d_tw2, tw2.size() * sizeof (float2)));
-    FX_CREATE (cudaMemcpy (e->d_tw1, tw1.data(), tw1.size() * sizeof (float2), cudaMemcpyHostToDevice));
     FX_CREATE (cudaMemcpy (e->d_tw2, tw2.data(), tw2.size() * sizeof (float2), cudaMemcpyHostToDevice));
     FX_CREATE (cudaMalloc (&e->d_tw1f, tw1f.size() * sizeof (float2)));
     FX_CREATE (cudaMemcpy (e->d_tw1f, tw1f.data(), tw1f.size() * sizeof (float2), cudaMemcpyHostToDevice));
@@ -912,8 +909,7 @@ fx_status analyse_host_pipeline (fx_engine* e, const unsigned char* src, long ro
     // Track groups: about fifty per call (the first group's upload and the last group's analysis are the only parts of
     // the pipeline that do not overlap), but never below ~64 MiB of fp32 audio -- small groups would have to cut every
     // track into short chunks to fill the GPU, and each chunk start refills a whole window
-    long want_groups = 48;
-    if (const char* env = getenv ("FXB200_PIPE_GROUPS")) { const long v = atol (env); if (v > 0) want_groups = v; }
+    const long want_groups = 48;
     long per = (T + want_groups - 1) / want_groups;
     const long per_min = (64L << 20) / (used * (long) sizeof (float));
     if (per < per_min) per = per_min;

@@ -15,29 +15,19 @@
 // k1 * ROW + 17 k2 + k3, and the time samples a transform starts from at tpos (n) = (n >> 8) * ROW + phys (n & 255).
 // Rows are 273 elements apart and 16-element groups inside a row are skewed by one (phys (a) = a + (a >> 4)): the row
 // accesses of stage 2, the column accesses of stage 3 and the readers of runs of consecutive bins are conflict free.
-// Twiddles come from small tables evaluated in double on the host and rounded to fp32 (as JUCE does); the stage-1
-// twiddle W_N^(m k1) is the product of two table entries, W_N^(16 mh k1) * W_N^(ml k1) with m = 16 mh + ml, which
-// keeps the tables at a few KB so that three CTAs fit on an SM.
-#pragma once
-#include <cuda_runtime.h>
-
-#ifndef FX_TW1_GLOBAL
-#define FX_TW1_GLOBAL 1     // 1: stage-1 twiddles from the full global table through L1 (one 8-byte load per twiddle, measured
-                            //    1.7 % faster); 0: product of two small shared-memory factors (two loads and a complex multiply)
-#endif
-
+// Twiddles come from tables evaluated in double on the host and rounded to fp32 (as JUCE does).  The stage-1 twiddles
+// W_N^(m k1) are read from a full global table through L1 (one 8-byte load per twiddle: 1.7 % faster than forming each one
+// from two small shared-memory factors); that table holds the fp32 products of the two factors, rounded as the in-line
+// product was (fx_tables.cu).
+//
 // Twiddle powers: only the twiddles W^1, W^2, W^4, W^8 of a thread are loaded (exact table values); the other eleven are
 // products of those, at most three multiplications deep (W^15 = W^8 W^4 W^2 W^1): 11 packed complex multiplies in place of 11
 // loads per stage and transform.  The loads ride the L1 / shared-memory data pipe, the busiest unit of the kernel, and the
 // stage-1 ones (global table through L1) expose their latency.  Measured (profiles/r02_v22_ab_*.txt), kernel ms at
 // N = 4096 / 2048 / 1024:  all loads 68.43 / 33.11 / 34.11;  stage 1 by powers 66.16 / 32.78 / 34.11;  stage 2 by powers
-// 68.14 / 33.51 / 34.23;  both 65.84 / 33.25 / 33.84.  Default: both stages at every size (see FX_TW2_POWERS below for N = 2048 / 1024).
-#ifndef FX_TW1_POWERS
-#define FX_TW1_POWERS 1                 // stage 1 (twiddles from the global table through L1)
-#endif
-#ifndef FX_TW2_POWERS
-#define FX_TW2_POWERS 1                 // stage 2 (twiddles from shared memory): 0 never, 1 always, 2 for R1 == 16 only.  At N = 2048 /
-#endif                                  // 1024 it costs ~1 % by itself and buys the shared memory for one more resident CTA (fx_analyse.cu)
+// 68.14 / 33.51 / 34.23;  both 65.84 / 33.25 / 33.84.  K1 takes both stages by powers at every size (fx_analyse.cu).
+#pragma once
+#include <cuda_runtime.h>
 
 namespace fx {
 
@@ -48,10 +38,6 @@ __device__ __forceinline__ int phys (int a) { return a + (a >> 4); }
 // instruction and a complex multiply two; ptxas folds the component swaps and negations of the operands below into
 // the instructions' operand modifiers (.LO_HI, .NP, .F32 broadcast).  The kernel is bound by issue slots, not by the
 // FP32 pipe: the packed forms halve the issue slots of the butterflies.
-#ifndef FX_F32X2
-#define FX_F32X2 1
-#endif
-#if FX_F32X2
 __device__ __forceinline__ float2 f2add (float2 a, float2 b)
 {
     float2 r;
@@ -80,12 +66,6 @@ __device__ __forceinline__ float2 f2fma (float2 a, float2 b, float2 c)
          : "=f"(r.x), "=f"(r.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y));
     return r;
 }
-#else
-__device__ __forceinline__ float2 f2add (float2 a, float2 b) { return make_float2 (a.x + b.x, a.y + b.y); }
-__device__ __forceinline__ float2 f2sub (float2 a, float2 b) { return make_float2 (a.x - b.x, a.y - b.y); }
-__device__ __forceinline__ float2 f2mul (float2 a, float2 b) { return make_float2 (__fmul_rn (a.x, b.x), __fmul_rn (a.y, b.y)); }
-__device__ __forceinline__ float2 f2fma (float2 a, float2 b, float2 c) { return make_float2 (fmaf (a.x, b.x, c.x), fmaf (a.y, b.y, c.y)); }
-#endif
 
 __device__ __forceinline__ float2 cadd (float2 a, float2 b) { return f2add (a, b); }
 __device__ __forceinline__ float2 csub (float2 a, float2 b) { return f2sub (a, b); }
@@ -203,21 +183,17 @@ template <int R1> struct FftDims
     static constexpr int Q1      = 16 / R1;            // stage-1 butterflies per thread
     static constexpr int ROW     = 273;                // 256 * 17 / 16 + 1: consecutive bins (consecutive k1) fall into different banks
     static constexpr int EX_LEN  = R1 * ROW;           // float2 elements in the exchange buffer
-    static constexpr int TW1_LEN = (R1 - 1) * 32;      // float2, tw1[(k1 - 1) * 32 + mh]      = W_N^(16 mh k1)   (mh < 16)
-                                                       //         tw1[(k1 - 1) * 32 + 16 + ml] = W_N^(ml k1)      (ml < 16)
     static constexpr int TW2_FULL = 15 * 16;           // float2, tw2[(k2 - 1) * 16 + n3]      = W_256^(n3 k2)
-    // stage-2 twiddles by powers: the shared-memory copy holds only the rows k2 = 1, 2, 4, 8 (in that order)
-    static constexpr bool TW2_POWERS = FX_TW2_POWERS == 1 || (FX_TW2_POWERS == 2 && R1 == 16);
-    static constexpr int TW2_LEN = TW2_POWERS ? 4 * 16 : TW2_FULL;
-    // ... and it lives in the 16-byte holes of the caller's skewed sample ring (fx_analyse.cu: one unused float4 behind every 32
-    // floats): element e = row * 16 + n3 sits in hole e / 2, slot e % 2, holes 36 floats = 18 float2 apart.  The 16 lanes of a
-    // half warp read 8 holes, i.e. 8 different 16-byte bank groups: conflict free like the dense table.
+    // stage-2 twiddles by powers: the shared-memory copy holds only the rows k2 = 1, 2, 4, 8 (in that order), and it lives in
+    // the 16-byte holes of the caller's skewed sample ring (fx_analyse.cu: one unused float4 behind every 32 floats): element
+    // e = row * 16 + n3 sits in hole e / 2, slot e % 2, holes 36 floats = 18 float2 apart.  The 16 lanes of a half warp read
+    // 8 holes, i.e. 8 different 16-byte bank groups: conflict free like the dense table.
     static constexpr int TW2_HOLE_ROW = 8 * 18;        // float2 distance between the rows k2 = 1, 2, 4, 8 of one n3
 };
 
 // Stage 1 on v (slot q * R1 + n1 = input n1 of butterfly q), then twiddle and store to ex.
 template <int R1, bool INV>
-__device__ __forceinline__ void fft_stage1_store (float2* v, int m0, float2* __restrict__ ex, const float2* __restrict__ tw1, const float2* __restrict__ tw1f)
+__device__ __forceinline__ void fft_stage1_store (float2* v, int m0, float2* __restrict__ ex, const float2* __restrict__ tw1f)
 {
     using D = FftDims<R1>;
     #pragma unroll
@@ -226,40 +202,25 @@ __device__ __forceinline__ void fft_stage1_store (float2* v, int m0, float2* __r
         butterfly<R1, INV> (v + q * R1);
         const int m = m0 + D::T * q;
         const int pm = phys (m);
-#if ! FX_TW1_GLOBAL
-        const int mh = m >> 4, ml = 16 + (m & 15);
-#endif
-#if FX_TW1_POWERS
         float2 wp[16];
         wp[1] = __ldg (&tw1f[m]); wp[2] = __ldg (&tw1f[256 + m]);
         if (R1 > 4) wp[4] = __ldg (&tw1f[3 * 256 + m]);
         if (R1 > 8) wp[8] = __ldg (&tw1f[7 * 256 + m]);
         twiddle_powers<R1> (wp);
-#endif
         #pragma unroll
         for (int s = 0; s < R1; ++s)
         {
             const int k1 = out_index<R1> (s);
             float2 val = v[q * R1 + s];
-            if (k1 > 0)
-            {
-#if FX_TW1_POWERS
-                const float2 w = wp[k1];
-#elif FX_TW1_GLOBAL
-                const float2 w = __ldg (&tw1f[(k1 - 1) * 256 + m]);
-#else
-                const float2 wa = tw1[(k1 - 1) * 32 + mh], wb = tw1[(k1 - 1) * 32 + ml];
-                const float2 w = make_float2 (wa.x * wb.x - wa.y * wb.y, wa.x * wb.y + wa.y * wb.x);
-#endif
-                val = cmulw<INV> (val, w);
-            }
+            if (k1 > 0) val = cmulw<INV> (val, wp[k1]);
             ex[k1 * D::ROW + pm] = val;
         }
     }
 }
 
-// Stage 2 in place (one 16-point butterfly per thread).  Caller syncs before and after.
-template <int R1, bool INV, bool POWERS = FftDims<R1>::TW2_POWERS>
+// Stage 2 in place (one 16-point butterfly per thread).  Caller syncs before and after.  POWERS: tw2 is the compact table
+// in the holes of the ring (see FftDims), else the full table tw2[(k2 - 1) * 16 + n3].
+template <int R1, bool INV, bool POWERS>
 __device__ __forceinline__ void fft_stage2 (int t, float2* __restrict__ ex, const float2* __restrict__ tw2)
 {
     using D = FftDims<R1>;
@@ -269,9 +230,8 @@ __device__ __forceinline__ void fft_stage2 (int t, float2* __restrict__ ex, cons
     #pragma unroll
     for (int n2 = 0; n2 < 16; ++n2) v[n2] = row[n2 * 17];
     butterfly<16, INV> (v);
-    constexpr bool kPowers = POWERS;                      // the table is then the compact one: rows k2 = 1, 2, 4, 8
     float2 wp[16];
-    if (kPowers)
+    if (POWERS)
     {
         const float2* th = tw2 + 18 * (n3 >> 1) + (n3 & 1);                                  // tw2: first hole of the ring
         wp[1] = th[0]; wp[2] = th[D::TW2_HOLE_ROW]; wp[4] = th[2 * D::TW2_HOLE_ROW]; wp[8] = th[3 * D::TW2_HOLE_ROW];
@@ -282,29 +242,7 @@ __device__ __forceinline__ void fft_stage2 (int t, float2* __restrict__ ex, cons
     {
         const int k2 = out_index<16> (s);
         float2 val = v[s];
-        if (k2 > 0) val = cmulw<INV> (val, kPowers ? wp[k2] : tw2[(k2 - 1) * 16 + n3]);
-        row[k2 * 17] = val;
-    }
-}
-
-// Stage 2 with its 15 twiddles already in registers (loaded by the caller BEFORE the block barrier that separates stage 1
-// from stage 2, while stage 1's values are dead and the registers free).
-template <int R1, bool INV>
-__device__ __forceinline__ void fft_stage2_tw (int t, float2* __restrict__ ex, const float2* tw)
-{
-    using D = FftDims<R1>;
-    const int k1 = t >> 4, n3 = t & 15;
-    float2* row = ex + k1 * D::ROW + n3;
-    float2 v[16];
-    #pragma unroll
-    for (int n2 = 0; n2 < 16; ++n2) v[n2] = row[n2 * 17];
-    butterfly<16, INV> (v);
-    #pragma unroll
-    for (int s = 0; s < 16; ++s)
-    {
-        const int k2 = out_index<16> (s);
-        float2 val = v[s];
-        if (k2 > 0) val = cmulw<INV> (val, tw[k2 - 1]);
+        if (k2 > 0) val = cmulw<INV> (val, POWERS ? wp[k2] : tw2[(k2 - 1) * 16 + n3]);
         row[k2 * 17] = val;
     }
 }
@@ -324,55 +262,6 @@ __device__ __forceinline__ void fft_stage3 (int t, float2* __restrict__ ex)
     __syncwarp();                                         // every thread of the row has read its column
     #pragma unroll
     for (int s = 0; s < 16; ++s) col[out_index<16> (s)] = v[s];
-}
-
-// EXPERIMENT (FX_STAGE23_SHFL=1, off by default): stages 2 and 3 with the 2 -> 3 exchange done by warp shuffles inside the
-// half warp instead of through shared memory -- the "warp-shuffle butterflies for the small stages" of BASELINE.json's
-// north_star.  The exchange is a 16 x 16 transpose over 16 lanes: four rounds (lane ^ 8, 4, 2, 1), each moving half of a
-// lane's 16 complex values = 64 shuffles of 32 bits per round pair... 128 SHFL + the selects that pick what to send and
-// where to put it, against 16 STS.64 + 16 LDS.64 for the shared-memory form.  Measured slower (DESIGN.md section 7); kept
-// so that the number can be reproduced.
-#ifndef FX_STAGE23_SHFL
-#define FX_STAGE23_SHFL 0
-#endif
-template <int R1, bool INV>
-__device__ __forceinline__ void fft_stage23_shfl (int t, float2* __restrict__ ex, const float2* __restrict__ tw2)
-{
-    using D = FftDims<R1>;
-    const int k1 = t >> 4, n3 = t & 15;
-    float2* row = ex + k1 * D::ROW + n3;
-    float2 v[16], u[16];
-    #pragma unroll
-    for (int n2 = 0; n2 < 16; ++n2) v[n2] = row[n2 * 17];
-    butterfly<16, INV> (v);
-    #pragma unroll
-    for (int s = 0; s < 16; ++s)
-    {
-        const int k2 = out_index<16> (s);
-        float2 val = v[s];
-        if (k2 > 0) val = cmulw<INV> (val, tw2[(k2 - 1) * 16 + n3]);
-        u[k2] = val;                                       // natural order: lane n3 holds Y_n3[k2], k2 = 0 .. 15
-    }
-    // transpose over the 16 lanes of the half warp: element (lane L, index I) moves to (lane I, index L)
-    #pragma unroll
-    for (int b = 8; b > 0; b >>= 1)
-    {
-        const bool up = (n3 & b) != 0;
-        #pragma unroll
-        for (int i = 0; i < 16; ++i)
-        {
-            if (i & b) continue;
-            const float2 send = up ? u[i] : u[i | b];
-            float2 recv;
-            recv.x = __shfl_xor_sync (0xffffffffu, send.x, b);
-            recv.y = __shfl_xor_sync (0xffffffffu, send.y, b);
-            if (up) u[i] = recv; else u[i | b] = recv;
-        }
-    }
-    butterfly<16, INV> (u);                                // lane k2 now holds Y_n3[k2] at index n3
-    float2* col = ex + k1 * D::ROW + n3 * 17;              // (this lane's k2 is its index in the half warp)
-    #pragma unroll
-    for (int s = 0; s < 16; ++s) col[out_index<16> (s)] = u[s];
 }
 
 // position of spectrum bin k / of time sample n in the exchange buffer (see the header comment)

@@ -5,20 +5,6 @@
 #include <stdint.h>
 #include "../../include/fx_engine.h"
 
-// pass 1's sums are reduced across the lanes of a warp in fp32 (1) or fp64 (0): K1 and K2 (the flux of a chunk's first
-// non-silent frame) must agree on it, see fx_analyse.cu
-#ifndef FX_P1SUM_F32
-#define FX_P1SUM_F32 1
-#endif
-// the inharmonicity sum and the mantissa of the flatness product's scan are fp32 across the lanes (fx_analyse.cu); with all
-// three on, every per-warp partial K1 hands to K1b is an fp32 value and the record stores it as one
-#ifndef FX_INHARM_F32
-#define FX_INHARM_F32 1
-#endif
-#ifndef FX_MESCAN_F32
-#define FX_MESCAN_F32 1
-#endif
-
 namespace fx {
 
 constexpr int kHistRows   = 32;   // raw feature rows carried between calls (10-tap smoothing + <=16-deep onset window + 5)
@@ -31,18 +17,15 @@ constexpr int kMaxOnsetHist = 16;
 // warp): K1 reduces across warps only what its own threads need (magnitude sum, maxima, the lag search), and no warp collects
 // the others' partials on its way into the next frame's first barrier (-2.4 % kernel time at N = 2048 / 1024, where the five
 // parts of the old record stage shared four / two warps).  K1b adds them in the order of the butterfly K1 used to run
-// (pairwise tree over the warps), so the features are the same bits.
-#if FX_P1SUM_F32 && FX_INHARM_F32 && FX_MESCAN_F32
-typedef float part_t;              // 64-byte WarpPart: the frame record is 272 / 400 / 656 bytes at N = 1024 / 2048 / 4096
-#else
-typedef double part_t;             // 96-byte WarpPart (336 / 528 / 912 bytes)
-#endif
+// (pairwise tree over the warps), so the features are the same bits.  Every partial is reduced across the lanes of its warp
+// in fp32 (pass 1's sums, the inharmonicity sum, the mantissa of the flatness product's scan), so the record stores it as one:
+// a 64-byte WarpPart, and a frame record of 272 / 400 / 656 bytes at N = 1024 / 2048 / 4096.
 struct alignas (16) WarpPart
 {
-    part_t p1[8];       // pass 1, the transposed butterfly's slots: S0 = sum mag, W1 = sum x mag, flux, low-energy sum, S2 = sum x^2 mag,
+    float  p1[8];       // pass 1, the transposed butterfly's slots: S0 = sum mag, W1 = sum x mag, flux, low-energy sum, S2 = sum x^2 mag,
                         // S4 = sum mag^2, gated sum, (unused)            (x = (bin + 1/2) / M)
-    part_t inharm;      // sum of f0Proportion * binMagnitude over the warp's peaks
-    part_t scan_m;      // extended-range product of the warp's gated magnitudes: mantissa in [0.5, 1] ...
+    float  inharm;      // sum of f0Proportion * binMagnitude over the warp's peaks
+    float  scan_m;      // extended-range product of the warp's gated magnitudes: mantissa in [0.5, 1] ...
     int    scan_e;      // ... and exponent
     int    count;       // gated bins
     int    npeaks;
@@ -55,7 +38,7 @@ struct alignas (16) FrameHead
     float  have_prev, lag, pitch_margin, peak_margin, flat_margin;
     float  her_mx[18];             // largest |Re A| around the 15 sub-octave and 3 harmonic bins of f0 (HarmonicCharacteristics.h:147-210), < 0: not used
 };
-static_assert ((sizeof (WarpPart) == 96 || sizeof (WarpPart) == 64) && sizeof (FrameHead) == 144, "the records are runs of 16-byte multiples (bulk copies in K1b)");
+static_assert (sizeof (WarpPart) == 64 && sizeof (FrameHead) == 144, "the records are runs of 16-byte multiples (bulk copies in K1b)");
 __host__ __device__ constexpr size_t frame_rec_bytes (int window) { return sizeof (FrameHead) + (size_t) (window / 512) * sizeof (WarpPart); }
 
 // ---- K1: per-(track, chunk) frame walker ------------------------------------------------------------
@@ -79,8 +62,7 @@ struct AnalyseParams
     double       sample_rate;
     double       bin_var;          // slope: sum ((i/M - 0.5)^2) / M evaluated on the host in the reference's order
     float        iir_c1, iir_c2;   // pi/2 and exp (-pi/2) in fp32 (RealTimeAudioAnalysis.h:122)
-    const float2* tw1;             // global twiddle tables (fx_fft.cuh layout)
-    const float2* tw2;
+    const float2* tw2;             // stage-2 twiddles, the full table (fx_fft.cuh layout): K1 copies the rows k2 = 1, 2, 4, 8
     const float2* tw1f;            // stage-1 twiddles in full, [(k1 - 1) * 256 + m] = W_N^(m k1) (the two-factor product, rounded as the kernel used to), read through L1
     // per-lag tables, slot lag = 1 .. window, slot 0 = "no lag found" (lag -1), evaluated on the host in the reference's own
     // double arithmetic from f0 = (nyquist * 2) / lag (PitchAnalyser.h:57):

@@ -106,7 +106,7 @@ __global__ void __launch_bounds__ (16 * R1) k_legacy_spectrum (const LegacyParam
             v[q * R1 + n1] = make_float2 (__fmul_rn (x, g), 0.0f);
         }
     __syncthreads();
-    fft_stage1_store<R1, false> (v, t, ex, nullptr, p.tw1f);
+    fft_stage1_store<R1, false> (v, t, ex, p.tw1f);
     __syncthreads();
     fft_stage2<R1, false, false> (t, ex, tw2);
     __syncwarp();
@@ -530,8 +530,8 @@ extern "C" fx_status fx_legacy_analyse_host (int device, int window, double samp
     float2 *d_tw1f = nullptr, *d_tw2 = nullptr;
     cudaStream_t s = nullptr;
     fx_status st = FX_ERR_CUDA;
-    std::vector<float2> tw1, tw2, tw1f;
-    build_twiddles (N, tw1, tw2, tw1f);
+    std::vector<float2> tw2, tw1f;
+    build_twiddles (N, tw2, tw1f);
     double bv = 0.0;                                                                        // :589-593 binVar, the reference's order
     for (double i = 0.0; i < (double) nb; i++) { const double ni = i / (double) nb; bv += (ni - 0.5) * (ni - 0.5); }
     bv /= (double) nb;

@@ -46,7 +46,7 @@ __global__ void __launch_bounds__ (256) k_flux_fix (const FluxFixParams p)
 
     // The sum runs in K1's own order and precision, so that a frame's flux does not depend on where the chunk boundaries fall
     // (tests: chunked, streamed and split calls are bit-identical): thread t takes bins 8 t .. 8 t + 7 in sequence (fp64), the
-    // lanes of a warp are added as K1's butterfly does (distances 1, 2, 4, 8, 16; in fp32 when K1 reduces pass 1 in fp32) and
+    // lanes of a warp are added as K1's butterfly does (distances 1, 2, 4, 8, 16; in fp32 like K1's) and
     // the warps as K1b's pairwise tree.  blockDim.x = M / 8 = the thread count of K1.
     double flux = 0.0;
     {
@@ -61,15 +61,10 @@ __global__ void __launch_bounds__ (256) k_flux_fix (const FluxFixParams p)
             if (diff > 0.0) flux += diff;                             // :77-79
         }
     }
-#if FX_P1SUM_F32
     float fl = (float) flux;
     #pragma unroll
     for (int off = 1; off < 32; off <<= 1) fl += __shfl_xor_sync (0xffffffffu, fl, off);
     flux = (double) fl;
-#else
-    #pragma unroll
-    for (int off = 1; off < 32; off <<= 1) flux += __shfl_xor_sync (0xffffffffu, flux, off);
-#endif
     if ((t & 31) == 0) wsum[t >> 5] = flux;
     __syncthreads();
     if (t == 0)

@@ -6,11 +6,12 @@
 namespace fx {
 
 // twiddle tables in the layout fx_fft.cuh expects; evaluated in double, rounded to fp32 (as juce::FFT does)
-void build_twiddles (int N, std::vector<float2>& tw1, std::vector<float2>& tw2, std::vector<float2>& tw1f)
+void build_twiddles (int N, std::vector<float2>& tw2, std::vector<float2>& tw1f)
 {
     const int R1 = N / 256;
     const double pi = 3.14159265358979323846;
-    tw1.assign ((size_t) (R1 - 1) * 32, make_float2 (1.0f, 0.0f));
+    // the two factors of a stage-1 twiddle: tw1[(k1 - 1) * 32 + mh] = W_N^(16 mh k1), tw1[(k1 - 1) * 32 + 16 + ml] = W_N^(ml k1)
+    std::vector<float2> tw1 ((size_t) (R1 - 1) * 32, make_float2 (1.0f, 0.0f));
     for (int k1 = 1; k1 < R1; ++k1)
         for (int i = 0; i < 16; ++i)
         {

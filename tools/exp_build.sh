@@ -1,6 +1,6 @@
 #!/bin/bash
 # Build kernel-experiment variants of libfxb200.so (never committed; lib/exp/ is git-ignored with every other .so):
-#   tools/exp_build.sh name '<extra nvcc flags, e.g. -DFX_SINGLE_PASS=0>' ['sed-script for csrc/fx_analyse.cu'] ['sed-script for fx_fft.cuh']
+#   tools/exp_build.sh name '<extra nvcc flags, e.g. -Xptxas -v>' ['sed-script for csrc/fx_analyse.cu'] ['sed-script for fx_fft.cuh']
 # -> feature-extractor_b200/lib/exp/libfxb200_<name>.so ; select it with FXB200_LIB=<path>
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
