@@ -276,6 +276,24 @@ __device__ __noinline__ void fft_core (V16 io, int m0)
     __syncwarp();                                           // rows are private to a half warp from here on
     fft_stage3<R1, false> (t, sm.ex);
 }
+// fft_core_pruned: the same transform for the parity-mode kernels, which call it for both transforms.  even (uniform): the input
+// is even and only the rows k1 <= R1 / 2 of the spectrum are computed (fx_fft.cuh); X[k] of the other rows is X[N - k], in a
+// computed row.  The half warps of the skipped rows leave after the block barrier; the row boundary splits a warp at every
+// window size, so the warp barriers name the row's half warp only.  A runtime flag rather than a second out-of-line copy:
+// with two copies in one kernel ptxas spills 24 bytes at N = 4096.
+template <int R1>
+__device__ __noinline__ void fft_core_pruned (V16 io, int m0, bool even)
+{
+    Smem<R1>& sm = *reinterpret_cast<Smem<R1>*> (fx_smem_raw);
+    const int t = threadIdx.x;
+    fft_stage1_store<R1, false, true> (io.v, m0, sm.ex, sm.tw1f, even);
+    __syncthreads();
+    if (even && (t >> 4) > R1 / 2) return;
+    const unsigned rowmask = 0xffffu << (t & 16);
+    fft_stage2<R1, false, true> (t, sm.ex, reinterpret_cast<const float2*> (sm.ring + 32));
+    __syncwarp (rowmask);                                   // rows are private to a half warp from here on
+    fft_stage3<R1, false> (t, sm.ex, rowmask);
+}
 
 // MG: also compute the decision margins (diagnostics, FX_DIAG_*_MARGIN).  They feed nothing: a call that does not ask for the
 // diagnostics runs the instantiation without them -- same features, bit for bit (tests/test_gpu_parity.py).
@@ -318,6 +336,10 @@ k_analyse (const AnalyseParams p)
     // Per window size (profiles/r02_v28b_ab_*.txt): the low-energy sum as the magnitude sum of the threads below the boundary
     // bin, only the thread that straddles it testing bins, pays at N >= 2048 and costs 0.8 % at N = 1024 (spills).
     constexpr bool kLhrRange = R1 >= 8;
+    // Per window size (profiles/r02_v35_even_beta_ab.txt): FFT-beta on the even part of the frame with the mirror rows of the
+    // spectrum skipped (parity mode only: the power mode reads Im A) pays 3.6 % at N = 4096 (80 registers, no spills).  At
+    // N = 2048 it pays 1.4 % but makes ptxas spill 8 bytes; at N = 1024 (one skipped row of four, 8 bytes of spills) it costs 3.0 %.
+    constexpr bool kEvenBeta = ! SP && R1 == 16;
 
     S& sm = *reinterpret_cast<S*> (fx_smem_raw);
     float* workf = reinterpret_cast<float*> (sm.ex);          // fp32 view, skewed index phys (n)
@@ -524,7 +546,8 @@ k_analyse (const AnalyseParams p)
                 io.v[q * R1 + n1] = sm.ex[n1 * D::ROW + phys (T * q + t)];                  // tpos (n1 * 256 + m)
         // no barrier: stage 1 is in place per thread (it stores to ex[k1 * ROW + phys (m)], exactly the slots
         // ex[n1 * ROW + phys (m)] this thread has just read)
-        fft_core<R1> (io, t);
+        if (kEvenBeta) fft_core_pruned<R1> (io, t, false);
+        else           fft_core<R1> (io, t);
         __syncthreads();                                            // Z[k] = B[k] + i C[k] is complete, at zpos (k)
 
         // previous non-silent spectrum of this thread's bins: issued now, consumed in pass 1 (L2 latency hidden by the split)
@@ -785,6 +808,10 @@ k_analyse (const AnalyseParams p)
         // Z = A + i D:  Re Z = Re A directly, and Im Z[s] + Im Z[N-s] = 2 D[s] because Im A is odd.  P is scaled by a
         // power of two that matches its L2 norm to the frame's (an fp32 FFT's rounding noise is relative to the L2 norm
         // of what it transforms): neither sequence's noise then rises above a small multiple of its own (the lag search is invariant to the scale, cnd = d^2 s / sum).
+        // Parity mode: nothing reads Im A, so the transform takes the even part of the frame, e[n] = (x[n] + x[(N - n) & (N - 1)]) / 2,
+        // in place of x: Re Z = FFT (e) = Re A, Im Z = 2^k D, and Z is even.  Only the rows k1 <= R1 / 2 of the spectrum are
+        // computed (fft_core_pruned); bins and lags of the other rows are read at N - k.  The power mode needs Im A and
+        // transforms x.
         {
             float pscale = 1.0f;
             if (psum_all > 0.0f && psum_all < 3.0e38f && rms_sum > 0.0)
@@ -800,7 +827,60 @@ k_analyse (const AnalyseParams p)
             const int rg = (int) ((a0 + t) >> 5) & (N / 32 - 1), rl = (int) ((a0 + t) & 31);
             const int pa_up = 36 * warp + lane;                                                   // sk32 (c + t) - 36 (c / 32)
             const int pa_dn = -36 * warp - lane - (lane ? 4 : 0);                                 // sk32 (N - c - t) - 36 ((N - c) / 32)
-            if (NB <= 4)
+            // parity mode: the mirror sample a0 + N - c - t of the ring, from the per-thread base a0 - t
+            const int rg2 = (int) ((a0 - t) >> 5) & (N / 32 - 1), rl2 = (int) ((a0 - t) & 31);
+            const float hg = 0.5f * gain;
+            if (kEvenBeta && NB <= 4)
+            {
+                // as below; the mirrors of quarter g lie in quarter 3 - g of the window, one wrapped base per quarter (ml), except
+                // that of c = g N / 4 for thread 0: sample (4 - g) N / 4 of the window, which thread 0 loads as its own sample of
+                // quarter (4 - g) mod 4
+                float xo[Q1 * R1];
+                #pragma unroll
+                for (int g = 0; g < 4; ++g)
+                {
+                    const float* rq = sm.ring + 36 * ((rg + g * (N / 128)) & (N / 32 - 1)) + rl;
+                    #pragma unroll
+                    for (int q = 0; q < Q1; ++q)
+                        #pragma unroll
+                        for (int i = 0; i < R1 / 4; ++i)
+                            xo[q * R1 + g * (R1 / 4) + i] = rq[36 * ((i * 256 + T * q) / 32)];
+                }
+                #pragma unroll
+                for (int g = 0; g < 4; ++g)
+                {
+                    const float* ml = sm.ring + 36 * ((rg2 + (4 - g) * (N / 128) - 1) & (N / 32 - 1)) + rl2;    // sample a0 - t + (4 - g) N / 4 - 32
+                    #pragma unroll
+                    for (int q = 0; q < Q1; ++q)
+                        #pragma unroll
+                        for (int i = 0; i < R1 / 4; ++i)
+                        {
+                            const int n1 = g * (R1 / 4) + i;
+                            const int c = n1 * 256 + T * q, cq = c - g * (N / 4);
+                            const int pidx = (c < M) ? pa_up + 36 * (c / 32) : pa_dn + 36 * ((N - c) / 32);
+                            float xm;
+                            if (cq != 0)     xm = ml[-36 * ((cq - 32) / 32)];
+                            else if (t != 0) xm = ml[36];
+                            else             xm = xo[((4 - g) & 3) * (R1 / 4)];
+                            io.v[q * R1 + n1] = f2mul (make_float2 (xo[q * R1 + n1] + xm, sm.pa[pidx]), make_float2 (hg, pscale));
+                        }
+                }
+            }
+            else if (kEvenBeta)
+            {
+                #pragma unroll
+                for (int q = 0; q < Q1; ++q)
+                    #pragma unroll
+                    for (int n1 = 0; n1 < R1; ++n1)
+                    {
+                        const int c = n1 * 256 + T * q;
+                        const int pidx = (c < M) ? pa_up + 36 * (c / 32) : pa_dn + 36 * ((N - c) / 32);
+                        const int ridx = 36 * ((rg + c / 32) & (N / 32 - 1)) + rl;
+                        const int midx = 36 * ((rg2 + (N - c) / 32) & (N / 32 - 1)) + rl2;
+                        io.v[q * R1 + n1] = f2mul (make_float2 (sm.ring[ridx] + sm.ring[midx], sm.pa[pidx]), make_float2 (hg, pscale));
+                    }
+            }
+            else if (NB <= 4)
             {
                 // the window starts at a multiple of the hop: with hop >= N / 4 the ring wraps at a multiple of N / 4 samples, never
                 // inside a quarter of the window -- one wrapped base per quarter, compile-time offsets inside it
@@ -836,7 +916,8 @@ k_analyse (const AnalyseParams p)
         }
         // No barrier here: stage 1 of the transform stores to this thread's own slots of the exchange buffer, which nobody
         // reads between the barrier above (the split is complete) and the barrier inside the transform.
-        fft_core<R1> (io, t);
+        if (kEvenBeta) fft_core_pruned<R1> (io, t, true);
+        else           fft_core<R1> (io, t);
         // (the record of this frame is written after the frame's last barrier, one part per warp)
         __syncthreads();
         // The flatness product's continuation (record stage, below) starts from the spectrum bins behind the earliest event
@@ -876,10 +957,22 @@ k_analyse (const AnalyseParams p)
             #pragma unroll
             for (int j = 0; j < 16; j += 2)
             {
-                // Z[s] + Z[N - s]: 2 * 2^k * D[s], two lags per instruction
-                const float2 za = make_float2 (sm.ex[zl_own + zrun<R1> (j)].y, sm.ex[zl_own + zrun<R1> (j + 1)].y);
-                const float2 zb = make_float2 (sm.ex[j == 0 ? zl_self : zl_mirror + zrun<R1> (16 - j)].y, sm.ex[zl_mirror + zrun<R1> (15 - j)].y);
-                const float2 d2 = f2add (za, zb);
+                float2 d2;
+                if (! kEvenBeta)
+                {
+                    // Z[s] + Z[N - s]: 2 * 2^k * D[s], two lags per instruction
+                    const float2 za = make_float2 (sm.ex[zl_own + zrun<R1> (j)].y, sm.ex[zl_own + zrun<R1> (j + 1)].y);
+                    const float2 zb = make_float2 (sm.ex[j == 0 ? zl_self : zl_mirror + zrun<R1> (16 - j)].y, sm.ex[zl_mirror + zrun<R1> (15 - j)].y);
+                    d2 = f2add (za, zb);
+                }
+                else
+                {
+                    // Im Z[s] = 2^k D[s] (half the value above: cnd and its margins do not depend on the scale); the row of lag
+                    // s = 16 t + j is j mod R1, and a lag in a row that was not computed reads its mirror N - s
+                    const int j1 = j + 1;
+                    d2 = make_float2 (sm.ex[(j & (R1 - 1)) > R1 / 2 ? zl_mirror + zrun<R1> (16 - j) : zl_own + zrun<R1> (j)].y,
+                                      sm.ex[(j1 & (R1 - 1)) > R1 / 2 ? zl_mirror + zrun<R1> (16 - j1) : zl_own + zrun<R1> (j1)].y);
+                }
                 if (MG) { dv[j] = d2.x; dv[j + 1] = d2.y; }
                 const float2 s2 = f2add (make_float2 (s0f, s0f), make_float2 ((float) j, (float) (j + 1)));
                 const float2 a2 = f2mul (f2mul (d2, d2), s2);                                     // s = 0 contributes 0
@@ -900,7 +993,14 @@ k_analyse (const AnalyseParams p)
                         const float imA = 0.5f * (zk.y - sm.ex[j == 0 ? zb_self : zb_mirror + zrun<R1> (8 - j)].y);
                         ra[j] = __fsqrt_rn (fmaf (zk.x, zk.x, __fmul_rn (imA, imA)));
                     }
-                    else ra[j] = sm.ex[zb_own + zrun<R1> (j)].x;
+                    else if (! kEvenBeta) ra[j] = sm.ex[zb_own + zrun<R1> (j)].x;
+                    else
+                    {
+                        // a bin in a row that was not computed reads its mirror N - k.  The row of bin b0 + j is j mod R1, except
+                        // at N = 4096, where the run of an odd thread covers rows 8 .. 15
+                        const bool mirror = R1 == 16 ? (j > 0 && (t & 1)) : (j & (R1 - 1)) > R1 / 2;
+                        ra[j] = sm.ex[mirror ? zb_mirror + zrun<R1> (8 - j) : zb_own + zrun<R1> (j)].x;
+                    }
                 }
                 *reinterpret_cast<float4*> (&sm.pa[pb0])     = make_float4 (ra[0], ra[1], ra[2], ra[3]);
                 *reinterpret_cast<float4*> (&sm.pa[pb0 + 4]) = make_float4 (ra[4], ra[5], ra[6], ra[7]);

@@ -175,6 +175,20 @@ __device__ __forceinline__ void twiddle_powers (float2* w)
     }
 }
 
+// the powers above R / 2 that twiddle_powers<R> forms and twiddle_powers<R / 2> does not (w[3] .. w[R/2] already filled)
+template <int R>
+__device__ __forceinline__ void twiddle_powers_upper (float2* w)
+{
+    if (R == 4) w[3] = cmulw<false> (w[2], w[1]);
+    if (R == 8) { w[5] = cmulw<false> (w[4], w[1]); w[6] = cmulw<false> (w[4], w[2]); w[7] = cmulw<false> (w[4], w[3]); }
+    if (R == 16)
+    {
+        w[9]  = cmulw<false> (w[8], w[1]); w[10] = cmulw<false> (w[8], w[2]); w[11] = cmulw<false> (w[8], w[3]);
+        w[12] = cmulw<false> (w[8], w[4]); w[13] = cmulw<false> (w[8], w[5]); w[14] = cmulw<false> (w[8], w[6]);
+        w[15] = cmulw<false> (w[8], w[7]);
+    }
+}
+
 // Shared-memory footprint helpers (in elements)
 template <int R1> struct FftDims
 {
@@ -192,8 +206,12 @@ template <int R1> struct FftDims
 };
 
 // Stage 1 on v (slot q * R1 + n1 = input n1 of butterfly q), then twiddle and store to ex.
-template <int R1, bool INV>
-__device__ __forceinline__ void fft_stage1_store (float2* v, int m0, float2* __restrict__ ex, const float2* __restrict__ tw1f)
+// PRUNABLE: a runtime flag even says that the input is even (z[(N - n) & (N - 1)] = z[n], real and imaginary parts alike), so
+// X[N - k] = X[k] and row R1 - k1 of the exchange buffer holds the mirrors of row k1.  Outputs k1 > R1 / 2 are then neither
+// twiddled nor stored, and with them go the twiddle powers above R1 / 2, which only those rows use; the caller skips stages 2
+// and 3 of those rows.  The flag is uniform, so this is one branch per butterfly.
+template <int R1, bool INV, bool PRUNABLE = false>
+__device__ __forceinline__ void fft_stage1_store (float2* v, int m0, float2* __restrict__ ex, const float2* __restrict__ tw1f, bool even = false)
 {
     using D = FftDims<R1>;
     #pragma unroll
@@ -206,14 +224,39 @@ __device__ __forceinline__ void fft_stage1_store (float2* v, int m0, float2* __r
         wp[1] = __ldg (&tw1f[m]); wp[2] = __ldg (&tw1f[256 + m]);
         if (R1 > 4) wp[4] = __ldg (&tw1f[3 * 256 + m]);
         if (R1 > 8) wp[8] = __ldg (&tw1f[7 * 256 + m]);
-        twiddle_powers<R1> (wp);
+        if (! PRUNABLE)
+        {
+            twiddle_powers<R1> (wp);
+            #pragma unroll
+            for (int s = 0; s < R1; ++s)
+            {
+                const int k1 = out_index<R1> (s);
+                float2 val = v[q * R1 + s];
+                if (k1 > 0) val = cmulw<INV> (val, wp[k1]);
+                ex[k1 * D::ROW + pm] = val;
+            }
+            continue;
+        }
+        twiddle_powers<R1 / 2> (wp);
         #pragma unroll
         for (int s = 0; s < R1; ++s)
         {
             const int k1 = out_index<R1> (s);
+            if (k1 > R1 / 2) continue;
             float2 val = v[q * R1 + s];
             if (k1 > 0) val = cmulw<INV> (val, wp[k1]);
             ex[k1 * D::ROW + pm] = val;
+        }
+        if (! even)
+        {
+            twiddle_powers_upper<R1> (wp);
+            #pragma unroll
+            for (int s = 0; s < R1; ++s)
+            {
+                const int k1 = out_index<R1> (s);
+                if (k1 <= R1 / 2) continue;
+                ex[k1 * D::ROW + pm] = cmulw<INV> (v[q * R1 + s], wp[k1]);
+            }
         }
     }
 }
@@ -248,9 +291,10 @@ __device__ __forceinline__ void fft_stage2 (int t, float2* __restrict__ ex, cons
 }
 
 // Stage 3 in place: X[k1 + R1 k2 + 16 R1 k3] replaces element (k2, n3 = k3) of row k1.  The caller has made the stage-2
-// stores of this half warp visible (__syncwarp).
+// stores of this half warp visible (__syncwarp).  rowmask: the lanes that run this stage together (at least the half warp
+// of the row; a caller whose other half warp skips the stage passes the half warp alone).
 template <int R1, bool INV>
-__device__ __forceinline__ void fft_stage3 (int t, float2* __restrict__ ex)
+__device__ __forceinline__ void fft_stage3 (int t, float2* __restrict__ ex, unsigned rowmask = 0xffffffffu)
 {
     using D = FftDims<R1>;
     const int k1 = t >> 4, k2 = t & 15;
@@ -259,7 +303,7 @@ __device__ __forceinline__ void fft_stage3 (int t, float2* __restrict__ ex)
     #pragma unroll
     for (int n3 = 0; n3 < 16; ++n3) v[n3] = col[n3];
     butterfly<16, INV> (v);
-    __syncwarp();                                         // every thread of the row has read its column
+    __syncwarp (rowmask);                                 // every thread of the row has read its column
     #pragma unroll
     for (int s = 0; s < 16; ++s) col[out_index<16> (s)] = v[s];
 }
