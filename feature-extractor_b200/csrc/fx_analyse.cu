@@ -22,8 +22,9 @@
 //              (PitchAnalyser.h:120), which is all that can reach the lag search (PitchAnalyser.h:163)
 // K1 leaves the per-frame sums in a FrameRec; K1b (one thread per frame) applies the scalar tail of the
 // reference (pow / log10 / sqrt, clamps, gates) so that no serial libm code sits inside the frame loop.
-// Every sum accumulates in fp64 per thread like the reference, and across the warps; across the 32 lanes of a warp the
-// partials (fp32-accurate squares of an fp32 spectrum) are added in fp32.  No tensor cores: nothing here is a GEMM.
+// Every sum accumulates in fp64 per thread like the reference, and across the warps; across the 32 lanes of a warp the raw
+// moments that K1b subtracts from each other stay fp64, the other partials (sums of positive terms) are added in fp32.
+// No tensor cores: nothing here is a GEMM.
 #include "fx_fft.cuh"
 #include "fx_kernels.cuh"
 #include <math.h>
@@ -667,13 +668,18 @@ k_analyse (const AnalyseParams p)
                 }
             }
             lprod = me_from (mprod); lprod.e += esum;
-            // the norm of P rides in the free eighth slot of the transposed butterfly (profiles/r02_v31_ab_psum_always_4096.txt)
-            float s8[8] = { (float) mag_sum, (float) weighted, (float) flux, (float) lhr, (float) s2, (float) s4, (float) flat_sum, psum };
-            warp_sum_t<8> (s8, lane);
+            // The raw moments cross the lanes in fp64: K1b's spread is S2 - 2 c W1 + c^2 S0, and on a narrowband frame that difference
+            // is ~1e-6 of its terms, so fp32 partials of S0, W1, S2 (relative rounding ~6e-8) would leave errors of the order of the
+            // spread itself.  S4 takes the fourth fp64 slot, which costs no extra exchange.  The sums of positive terms that feed
+            // nothing but a ratio stay fp32; the norm of P rides in their free fourth slot (profiles/r02_v31_ab_psum_always_4096.txt).
+            double sd[4] = { mag_sum, weighted, s2, s4 };
+            float sf[4] = { (float) flux, (float) lhr, (float) flat_sum, psum };
+            warp_sum_t<4> (sd, lane);
+            warp_sum_t<4> (sf, lane);
             const int wcount = warp_addi (count);
             const float wmax = warp_max_nonneg (maxre);
             const float wraw = warp_max_nonneg (rawmax);
-            const float wps = __shfl_sync (0xffffffffu, s8[0], 7);                                  // slot 7's total lives in lanes = 7 mod 8
+            const float wps = __shfl_sync (0xffffffffu, sf[0], 3);                                  // slot 3's total lives in lanes = 3 mod 4
             float wmar = 1.0f;
             if (MG) wmar = warp_min_nonneg (fminf (gate_d * gate_inv, 0.5f));
             // inclusive warp scan of the extended-range product, in bin order; the mantissa in fp32 (the exponent is an integer,
@@ -694,22 +700,23 @@ k_analyse (const AnalyseParams p)
             ME exc; exc.m = __shfl_up_sync (0xffffffffu, inc.m, 1); exc.e = __shfl_up_sync (0xffffffffu, inc.e, 1);
             if (lane == 0) exc = me_one();
             lprod = exc;                                                                         // lane-exclusive prefix within the warp
-            // The warp's partials leave for K1b from here (the frame record's WarpPart of this warp, one 32-byte run); only what this CTA's own
+            // The warp's partials leave for K1b from here (the frame record's WarpPart of this warp, one 80-byte run); only what this CTA's own
             // threads need -- the magnitude sum, the largest |Re|, the norm of P and the product's warp totals -- also goes
-            // through shared memory.  After the transposed butterfly lane l < 8 holds the warp total of value warp_sum_slot<8> (l):
-            // 0 S0, 1 W1, 2 flux, 3 lhr, 4 S2, 5 S4, 6 flat_sum (7: zero).
+            // through shared memory.  After the transposed butterflies lane l holds the warp totals of slot warp_sum_slot<4> (l) of both
+            // arrays: sd 0 S0, 1 W1, 2 S2, 3 S4; sf 0 flux, 1 lhr, 2 flat_sum, 3 the norm of P (not recorded).
             WarpPart* wp = &rec_w[warp];
             if (lane == 31)
             {
                 *reinterpret_cast<double2*> (&sm.scan[warp]) = make_double2 (inc.m, __hiloint2double (__float_as_int ((float) inc.m), inc.e));
                 wp->scan_m = inc.m; wp->scan_e = inc.e;
             }
-            if (lane < 8) wp->p1[warp_sum_slot<8> (lane)] = (double) s8[0];
+            if (lane < 4) wp->p1d[warp_sum_slot<4> (lane)] = sd[0];
+            else if (lane < 7) wp->p1f[warp_sum_slot<4> (lane)] = sf[0];
             if (lane == 0)
             {
                 wp->count = wcount; wp->rawmax = wraw;
                 // S0: every thread needs the magnitude sum
-                *reinterpret_cast<double2*> (&sm.p1s[warp]) = make_double2 ((double) s8[0], __hiloint2double (__float_as_int (wps), __float_as_int (wmax)));
+                *reinterpret_cast<double2*> (&sm.p1s[warp]) = make_double2 (sd[0], __hiloint2double (__float_as_int (wps), __float_as_int (wmax)));
                 if (MG) sm.fmins[0][warp] = wmar;
             }
         }
@@ -1407,8 +1414,8 @@ k_analyse (const AnalyseParams p)
 
 // ---------------------------------------------------------------------------------------------------------
 // K1b: the scalar tail of both analyser bodies, one thread per frame, one warp per batch of 32 consecutive frames.
-// A batch's records are one contiguous run of 32 * frame_rec_bytes (8.5 .. 20.5 KB): it arrives in shared memory by ONE
-// bulk copy (a thread reading its own 272 .. 656-byte record straight from global memory touches a different sector with
+// A batch's records are one contiguous run of 32 * frame_rec_bytes (9.5 .. 24.5 KB): it arrives in shared memory by ONE
+// bulk copy (a thread reading its own 304 .. 784-byte record straight from global memory touches a different sector with
 // every load).  The tail is a long dependent fp64 chain (pow, five log10, three sqrt), so it needs many resident warps, and
 // the staged records would cap them: a block of 12 warps therefore shares THREE staging buffers in turn.  Warp w waits for
 // its batch in buffer w % 3, reduces the per-warp partials of its 32 frames into registers, hands the buffer to batch
@@ -1468,9 +1475,9 @@ __global__ void __launch_bounds__ (kFinalizeRows, kFzBlocks) k_finalize (const F
             for (int w = 0; w < NW; w += 2 * half) v[w] += v[w + half];
         return v[0];
     };
-    const double w1 = tree ([&] (int w) { return rw[w].p1[1]; }), flux = tree ([&] (int w) { return rw[w].p1[2]; });
-    const double lhr = tree ([&] (int w) { return rw[w].p1[3]; }), s2 = tree ([&] (int w) { return rw[w].p1[4]; });
-    const double s4 = tree ([&] (int w) { return rw[w].p1[5]; }), flat_sum = tree ([&] (int w) { return rw[w].p1[6]; });
+    const double w1 = tree ([&] (int w) { return rw[w].p1d[1]; }), s2 = tree ([&] (int w) { return rw[w].p1d[2]; });
+    const double s4 = tree ([&] (int w) { return rw[w].p1d[3]; }), flux = tree ([&] (int w) { return rw[w].p1f[0]; });
+    const double lhr = tree ([&] (int w) { return rw[w].p1f[1]; }), flat_sum = tree ([&] (int w) { return rw[w].p1f[2]; });
     const double inharm = tree ([&] (int w) { return rw[w].inharm; });
     int count_i = 0, npeaks_i = 0;
     float rawmax = 0.0f;

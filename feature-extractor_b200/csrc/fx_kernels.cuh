@@ -13,17 +13,18 @@ constexpr int kMaxOnsetHist = 16;
 
 // What K1 leaves for K1b (k_finalize) per frame: a FrameHead followed by one WarpPart per warp of the K1 CTA (window / 512 of
 // them), frame_rec_bytes (window) per frame.  fp64 wherever the reference accumulates in double.
-// The sums that only K1b looks at leave K1 as PER-WARP partials, stored by each warp where it forms them (one 64-byte run per
+// The sums that only K1b looks at leave K1 as PER-WARP partials, stored by each warp where it forms them (one 80-byte run per
 // warp): K1 reduces across warps only what its own threads need (magnitude sum, maxima, the lag search), and no warp collects
 // the others' partials on its way into the next frame's first barrier (-2.4 % kernel time at N = 2048 / 1024, where the five
 // parts of the old record stage shared four / two warps).  K1b adds them in the order of the butterfly K1 used to run
-// (pairwise tree over the warps), so the features are the same bits.  Every partial is reduced across the lanes of its warp
-// in fp32 (pass 1's sums, the inharmonicity sum, the mantissa of the flatness product's scan), so the record stores it as one:
-// a 64-byte WarpPart, and a frame record of 272 / 400 / 656 bytes at N = 1024 / 2048 / 4096.
+// (pairwise tree over the warps), so the features are the same bits.  The raw moments of pass 1 cross the lanes of their warp
+// in fp64, because K1b's spread is a cancelling difference of them (fx_analyse.cu); the other partials (flux, low-energy and
+// gated sums, the inharmonicity sum, the mantissa of the flatness product's scan) are reduced in fp32 and stored as such: an
+// 80-byte WarpPart, and a frame record of 304 / 464 / 784 bytes at N = 1024 / 2048 / 4096.
 struct alignas (16) WarpPart
 {
-    float  p1[8];       // pass 1, the transposed butterfly's slots: S0 = sum mag, W1 = sum x mag, flux, low-energy sum, S2 = sum x^2 mag,
-                        // S4 = sum mag^2, gated sum, (unused)            (x = (bin + 1/2) / M)
+    double p1d[4];      // pass 1, fp64 slots: S0 = sum mag, W1 = sum x mag, S2 = sum x^2 mag, S4 = sum mag^2     (x = (bin + 1/2) / M)
+    float  p1f[3];      // pass 1, fp32 slots: flux, low-energy sum, gated sum
     float  inharm;      // sum of f0Proportion * binMagnitude over the warp's peaks
     float  scan_m;      // extended-range product of the warp's gated magnitudes: mantissa in [0.5, 1] ...
     int    scan_e;      // ... and exponent
@@ -38,7 +39,7 @@ struct alignas (16) FrameHead
     float  have_prev, lag, pitch_margin, peak_margin, flat_margin;
     float  her_mx[18];             // largest |Re A| around the 15 sub-octave and 3 harmonic bins of f0 (HarmonicCharacteristics.h:147-210), < 0: not used
 };
-static_assert (sizeof (WarpPart) == 64 && sizeof (FrameHead) == 144, "the records are runs of 16-byte multiples (bulk copies in K1b)");
+static_assert (sizeof (WarpPart) == 80 && sizeof (FrameHead) == 144, "the records are runs of 16-byte multiples (bulk copies in K1b)");
 __host__ __device__ constexpr size_t frame_rec_bytes (int window) { return sizeof (FrameHead) + (size_t) (window / 512) * sizeof (WarpPart); }
 
 // ---- K1: per-(track, chunk) frame walker ------------------------------------------------------------

@@ -9,6 +9,7 @@ import pytest
 
 import oracle_util as ou
 import power_oracle
+from f64_features import bartlett_f32
 
 SR, N, H = 48000.0, 2048, 1024
 
@@ -49,21 +50,6 @@ def test_power_mode_is_phase_invariant_on_a_steady_tone(port, re_port):
     assert spread[1]["slope"] < 2e-6, spread
     # Re^2 mode flickers over the same frames (by three orders of magnitude more): the test fails if the mode is ignored
     assert spread[0]["her"] > 0.01 and spread[0]["inharm"] > 0.01 and spread[0]["slope"] > 1e-3, spread
-
-
-def bartlett_f32(x):
-    """RealTimeWindower::scaleBufferWithBartlettWindowing as the port applies it (gain accumulated in fp32)"""
-    half = len(x) // 2
-    w = np.empty(len(x), np.float32)
-    g, inc = np.float32(0.0), np.float32(1.0) / np.float32(half)
-    for i in range(half):
-        w[i] = g
-        g = np.float32(g + inc)
-    g, inc = np.float32(1.0), np.float32(-1.0) / np.float32(half)
-    for i in range(half):
-        w[half + i] = g
-        g = np.float32(g + inc)
-    return (x * w).astype(np.float32)
 
 
 def test_spectral_features_match_a_float64_restatement(port, re_port):
