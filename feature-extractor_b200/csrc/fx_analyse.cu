@@ -313,7 +313,9 @@ static_assert (kCtasR4 * (sizeof (Smem<4>) + 1024) <= 233472, "resident CTAs of 
 // pass.  Everything downstream squares or compares these values exactly as it squares and compares Re, so the two
 // places that form them (the split after FFT-alpha, the hand-over of A after FFT-beta) are the only branches on SP;
 // the instantiations without it are the parity mode, unchanged.
-template <int R1, bool MG, bool SP>
+// SO: the spectrum export (fx_analyse_device_spectrum).  Each frame's mag[m] = cr[m]^2, the per-bin energy the spectral pass
+// reads, is also stored to p.spec; the instantiations without it compile to the same instructions as before SO existed.
+template <int R1, bool MG, bool SP, bool SO>
 __global__ void __launch_bounds__ (16 * R1, (R1 == 16 ? kCtasR16 : (R1 == 8 ? kCtasR8 : kCtasR4)))
 k_analyse (const AnalyseParams p)
 {
@@ -593,6 +595,15 @@ k_analyse (const AnalyseParams p)
             *reinterpret_cast<float4*> (&sm.pa[pb0])     = make_float4 (pq[0], pq[1], pq[2], pq[3]);
             *reinterpret_cast<float4*> (&sm.pa[pb0 + 4]) = make_float4 (pq[4], pq[5], pq[6], pq[7]);
             if (t == 0) { const float cm = 2.0f * sm.ex[zpos<R1> (M)].y; sm.pa[sk32 (M)] = __fmul_rn (cm, cm); }      // C[N/2] is real and pairs with itself
+            if constexpr (SO)
+            {
+                // mag[b0 + j] rounded once to fp32 (pass 1 squares the same cr[j] exactly in fp64), every frame, silent or not.
+                // Two 16-byte stores per thread, 1 KB contiguous per warp; evict-first (st.global.cs), so that the rows
+                // streaming out do not push the stage-1 twiddle table (read through L1 / L2 every frame) out of the caches.
+                float4* row = reinterpret_cast<float4*> (p.spec + (size_t) (track * p.n_frames + f) * M + b0);
+                __stcs (row,     make_float4 (__fmul_rn (cr[0], cr[0]), __fmul_rn (cr[1], cr[1]), __fmul_rn (cr[2], cr[2]), __fmul_rn (cr[3], cr[3])));
+                __stcs (row + 1, make_float4 (__fmul_rn (cr[4], cr[4]), __fmul_rn (cr[5], cr[5]), __fmul_rn (cr[6], cr[6]), __fmul_rn (cr[7], cr[7])));
+            }
         }
 
         // RMS (RealTimeAnalyser.h:207-208)
@@ -1608,33 +1619,46 @@ __global__ void __launch_bounds__ (kFinalizeRows, kFzBlocks) k_finalize (const F
 }
 
 // ---------------------------------------------------------------------------------------------------------
+template <int R1, bool SO> static void launch_so (unsigned g, const AnalyseParams& p, cudaStream_t stream)
+{
+    const unsigned nt = 16 * R1;
+    const size_t smem = sizeof (Smem<R1>);
+    if (p.spectrum == FX_SPECTRUM_POWER)
+    {
+        if (p.want_margins) k_analyse<R1, true, true, SO><<<g, nt, smem, stream>>> (p);
+        else                k_analyse<R1, false, true, SO><<<g, nt, smem, stream>>> (p);
+    }
+    else
+    {
+        if (p.want_margins) k_analyse<R1, true, false, SO><<<g, nt, smem, stream>>> (p);
+        else                k_analyse<R1, false, false, SO><<<g, nt, smem, stream>>> (p);
+    }
+}
+
 template <int R1> static cudaError_t launch_t (long n_tracks, const AnalyseParams& p, cudaStream_t stream)
 {
     const long grid = n_tracks * p.n_chunks;
     if (grid <= 0) return cudaSuccess;
-    const unsigned g = (unsigned) grid, nt = 16 * R1;
-    const size_t smem = sizeof (Smem<R1>);
-    if (p.spectrum == FX_SPECTRUM_POWER)
-    {
-        if (p.want_margins) k_analyse<R1, true, true><<<g, nt, smem, stream>>> (p);
-        else                k_analyse<R1, false, true><<<g, nt, smem, stream>>> (p);
-    }
-    else
-    {
-        if (p.want_margins) k_analyse<R1, true, false><<<g, nt, smem, stream>>> (p);
-        else                k_analyse<R1, false, false><<<g, nt, smem, stream>>> (p);
-    }
+    if (p.spec) launch_so<R1, true> ((unsigned) grid, p, stream);
+    else        launch_so<R1, false> ((unsigned) grid, p, stream);
     return cudaGetLastError();
+}
+
+template <int R1, bool SO> static cudaError_t configure_so()
+{
+    const int smem = (int) sizeof (Smem<R1>);
+    cudaError_t ce = cudaFuncSetAttribute (k_analyse<R1, true, false, SO>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, false, false, SO>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, true, true, SO>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, false, true, SO>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    return ce;
 }
 
 template <int R1> static cudaError_t configure_t()
 {
-    const int smem = (int) sizeof (Smem<R1>);
     cudaError_t ce = cudaFuncSetAttribute (k_finalize<R1 / 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (kFzBufs * 32 * frame_rec_bytes (256 * R1)));
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute (k_analyse<R1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (ce == cudaSuccess) ce = configure_so<R1, false>();
+    if (ce == cudaSuccess) ce = configure_so<R1, true>();
     return ce;
 }
 

@@ -257,7 +257,7 @@ int choose_chunks (const fx_engine* e, long n_tracks, long frames)
 // offset to track t0 as well (rec: t0 * frames, chunk buffers: t0 * n_chunks).  Does NOT advance the bookkeeping.
 fx_status run_range (fx_engine* e, int t0, int nt, int n_chunks, int flip, long frames_done, const fx_scratch& sc,
                      const float* d_audio, long track_stride, long frames,
-                     float* d_raw, float* d_smooth, float* d_diag, float* d_latest, cudaStream_t s, bool may_profile)
+                     float* d_raw, float* d_smooth, float* d_diag, float* d_spec, float* d_latest, cudaStream_t s, bool may_profile)
 {
     const int in = flip, out = flip ^ 1;
     const int fpc = (int) ((frames + n_chunks - 1) / n_chunks);
@@ -279,6 +279,7 @@ fx_status run_range (fx_engine* e, int t0, int nt, int n_chunks, int flip, long 
     a.rec = sc.rec;
     a.first_spec = sc.first_spec; a.last_spec = sc.last_spec; a.first_idx = sc.first_idx;
     a.spectrum = e->cfg.spectrum;
+    a.spec = d_spec;
     const bool prof = may_profile && e->profiling;
     fx_engine::ProfRec pr{};
     if (prof)
@@ -496,7 +497,7 @@ fx_status rt_issue (fx_engine* e, fx_group& g, long* hops_out)
     int n_chunks = choose_chunks (e, g.n, hops);
     if (n_chunks > g.max_chunks) n_chunks = g.max_chunks;
     fx_status st = run_range (e, g.t0, g.n, n_chunks, g.flip, g.frames_done, g.scratch, g.d_stage, n, hops, g.d_raw, g.d_smooth,
-                              nullptr, e->d_latest + (size_t) g.t0 * kLatestWords, g.stream, false);
+                              nullptr, nullptr, e->d_latest + (size_t) g.t0 * kLatestWords, g.stream, false);
     if (st != FX_OK) return st;
     FX_CUDA (e, cudaMemcpyAsync (g.h_latest, e->d_latest + (size_t) g.t0 * kLatestWords,
                                   (size_t) g.n * kLatestWords * sizeof (float), cudaMemcpyDeviceToHost, g.stream));
@@ -863,20 +864,26 @@ fx_status fx_reset (fx_engine* e)
 }
 
 // ---- offline / batch analysis ------------------------------------------------------------------------------------
-fx_status fx_analyse_device (fx_engine* e, const float* d_audio, long track_stride, long n_samples,
-                             float* d_raw, float* d_smooth, float* d_diag, void* stream, long* n_frames)
+fx_status fx_analyse_device_spectrum (fx_engine* e, const float* d_audio, long track_stride, long n_samples,
+                                      float* d_raw, float* d_smooth, float* d_diag, float* d_spec, void* stream, long* n_frames)
 {
     if (! e || ! d_audio || n_samples < 0 || track_stride < n_samples) return FX_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> api (e->api_mutex);
+    if (((uintptr_t) d_spec & 15u) != 0) { set_error (e, "d_spec must be 16-byte aligned"); return FX_ERR_INVALID_ARG; }      // K1 stores 16-byte vectors
     FX_CUDA (e, cudaSetDevice (e->cfg.device));
     cudaStream_t s = stream ? (cudaStream_t) stream : e->stream;
     const long frames = n_samples / e->H;
     if (n_frames) *n_frames = frames;
     if (frames == 0) return FX_OK;
     if (frames > 0x7fffffffL / (FX_NUM_FEATURES * 4)) { set_error (e, "too many frames in one call"); return FX_ERR_INVALID_ARG; }
+    const long T = e->cfg.n_tracks;
+    // K1 indexes the spectrum rows in 64 bits: T * frames * M floats must have a byte size that a long holds
+    if (d_spec && T * frames > 0x7fffffffffffffffL / ((long) e->M * (long) sizeof (float)))
+    {
+        set_error (e, "the spectrum output is too large for one call"); return FX_ERR_INVALID_ARG;
+    }
     fx_status st = offline_begin (e, s);
     if (st != FX_OK) return st;
-    const long T = e->cfg.n_tracks;
     const int n_chunks = choose_chunks (e, T, frames);
     st = ensure_chunks (e, T * n_chunks);
     if (st != FX_OK) return st;
@@ -889,9 +896,15 @@ fx_status fx_analyse_device (fx_engine* e, const float* d_audio, long track_stri
         d_raw = e->d_raw;
     }
     st = run_range (e, 0, (int) T, n_chunks, e->groups[0]->flip, e->groups[0]->frames_done, offline_scratch (e, 0, frames, n_chunks),
-                    d_audio, track_stride, frames, d_raw, d_smooth, d_diag, e->d_latest, s, true);
+                    d_audio, track_stride, frames, d_raw, d_smooth, d_diag, d_spec, e->d_latest, s, true);
     if (st != FX_OK) return st;
     return offline_end (e, s, frames);
+}
+
+fx_status fx_analyse_device (fx_engine* e, const float* d_audio, long track_stride, long n_samples,
+                             float* d_raw, float* d_smooth, float* d_diag, void* stream, long* n_frames)
+{
+    return fx_analyse_device_spectrum (e, d_audio, track_stride, n_samples, d_raw, d_smooth, d_diag, nullptr, stream, n_frames);
 }
 
 namespace {
@@ -1002,7 +1015,7 @@ fx_status analyse_host_pipeline (fx_engine* e, const unsigned char* src, long ro
         float* ds = e->d_smooth + roff * FX_NUM_FEATURES;
         float* dd = e->d_diag + roff * FX_NUM_DIAG;
         st = run_range (e, (int) t0, (int) nt, n_chunks, flip, frames_done, offline_scratch (e, t0, frames, n_chunks),
-                        e->d_audio_slot[slot], used, frames, dr, smooth ? ds : nullptr, diag ? dd : nullptr,
+                        e->d_audio_slot[slot], used, frames, dr, smooth ? ds : nullptr, diag ? dd : nullptr, nullptr,
                         e->d_latest + (size_t) t0 * kLatestWords, s_run, true);
         if (st != FX_OK) return st;
         mark (s_run);

@@ -79,6 +79,8 @@ struct AnalyseParams
     float*       last_spec;        // [n_tracks][n_chunks][M]  ... of its last non-silent frame
     int*         first_idx;        // [n_tracks][n_chunks]     frame index of the first non-silent frame, -1 if none
     int          spectrum;         // fx_config::spectrum: FX_SPECTRUM_RE_SQUARED or FX_SPECTRUM_POWER (selects the instantiation)
+    // (last, so that the offsets of the fields above -- and the instructions of the kernels without it -- stay as they were)
+    float*       spec;             // [n_tracks][n_frames][M] mag[m] of every frame, 16-byte aligned, 64-bit row index; null: not exported (selects the instantiation)
 };
 
 int         analyse_ctas_per_sm (int window);      // resident CTAs per SM k_analyse is compiled for (chunk heuristic)

@@ -34,7 +34,7 @@ EXPORTS = (
     "fx_pcm_bytes_per_sample", "fx_analyse_host_pcm", "fx_decode_pcm_device",
     "fx_poll_block", "fx_rt_start", "fx_rt_stop", "fx_set_features_callback", "fx_set_track_active", "fx_clear_buffer",
     "fx_set_sample_rate", "fx_rt_get_stats", "fx_osc_encode_tracks", "fx_synth_device_at", "fx_h2d_probe",
-    "fx_legacy_analyse_host",
+    "fx_legacy_analyse_host", "fx_analyse_device_spectrum",
 )
 
 # fx_engine.h FX_LEGACY_*: output slots of the legacy offline analyser (AudioAnalysis.h)
@@ -101,6 +101,9 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
     lib.fx_analyse_host.restype = c_int
     lib.fx_analyse_device.argtypes = [c_void_p, c_void_p, c_long, c_long, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(c_long)]
     lib.fx_analyse_device.restype = c_int
+    lib.fx_analyse_device_spectrum.argtypes = [c_void_p, c_void_p, c_long, c_long, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                               POINTER(c_long)]
+    lib.fx_analyse_device_spectrum.restype = c_int
     lib.fx_push_block.argtypes = [c_void_p, c_int, c_int, POINTER(c_void_p), c_int]
     lib.fx_push_block.restype = c_int
     lib.fx_process.argtypes = [c_void_p, POINTER(c_long)]
@@ -284,11 +287,18 @@ class Engine:
 
     # -- batch analysis, device buffers (raw pointers; torch is only used by callers for allocation) ----------
     def analyse_device(self, d_audio_ptr: int, track_stride: int, n_samples: int, d_raw_ptr=None, d_smooth_ptr=None,
-                       d_diag_ptr=None, stream: int | None = None) -> int:
+                       d_diag_ptr=None, stream: int | None = None, d_spec_ptr=None) -> int:
+        """d_spec_ptr: device buffer of [n_tracks][frames][window // 2] fp32 (16-byte aligned) that receives the spectrum the
+        spectral features read (fx_analyse_device_spectrum); None: no spectrum."""
         nf = c_long(0)
-        st = self.lib.fx_analyse_device(self._h, d_audio_ptr, track_stride, n_samples, d_raw_ptr, d_smooth_ptr,
-                                        d_diag_ptr, stream, ctypes.byref(nf))
-        self._check(st, "fx_analyse_device")
+        if d_spec_ptr is None:
+            st = self.lib.fx_analyse_device(self._h, d_audio_ptr, track_stride, n_samples, d_raw_ptr, d_smooth_ptr,
+                                            d_diag_ptr, stream, ctypes.byref(nf))
+            self._check(st, "fx_analyse_device")
+        else:
+            st = self.lib.fx_analyse_device_spectrum(self._h, d_audio_ptr, track_stride, n_samples, d_raw_ptr, d_smooth_ptr,
+                                                     d_diag_ptr, d_spec_ptr, stream, ctypes.byref(nf))
+            self._check(st, "fx_analyse_device_spectrum")
         return nf.value
 
     def synth_device(self, d_audio_ptr: int, track_stride: int, n_samples: int, first_track: int = 0, seed: int = 0x5EED,

@@ -139,6 +139,21 @@ fx_status   fx_analyse_host   (fx_engine* e, const float* audio, long track_stri
 fx_status   fx_analyse_device (fx_engine* e, const float* d_audio, long track_stride, long n_samples,
                                float* d_raw, float* d_smooth, float* d_diag, void* stream, long* n_frames);
 
+/* fx_analyse_device_spectrum: fx_analyse_device that also writes the spectrum the spectral features are computed from.
+ * d_spec is DEVICE memory, [n_tracks][frames][window / 2] fp32, contiguous: 2 * window bytes per track and frame (15.7 GB
+ * for 4096 tracks x 10 s at 48 kHz, N = 4096, H = 1024).  Row (t, f), bin m = 0 .. window/2 - 1 holds mag[m], the value
+ * SpectralCharacteristics.h:68-73 reads for frame f, rounded once to fp32:
+ *   FX_SPECTRUM_RE_SQUARED  (Re X[m])^2
+ *   FX_SPECTRUM_POWER       |X[m]|^2
+ * where X is the transform of the Bartlett-windowed frame with the gain applied (after a gain change the older part of the
+ * window keeps its old gain, as for the features).  Every frame is written, the ones the 0.05 magnitude gate silences and
+ * the zero-padded start of a stream included.  d_spec must be 16-byte aligned (FX_ERR_INVALID_ARG otherwise, nothing
+ * written); d_spec = NULL is fx_analyse_device.  The output is device-only: copying it to the host would take several
+ * times as long as the analysis. */
+fx_status   fx_analyse_device_spectrum (fx_engine* e, const float* d_audio, long track_stride, long n_samples,
+                                        float* d_raw, float* d_smooth, float* d_diag, float* d_spec,
+                                        void* stream, long* n_frames);
+
 /* ---- file ingest: PCM in, features out ---------------------------------------------------------------
  * Replaces the file route of the reference: AudioFilePlayer::loadFileIntoTransport (AudioFilePlayer.h:41-60) hands the
  * file to JUCE's format readers, the transport plays it through the device output and AudioDataCollector re-captures one

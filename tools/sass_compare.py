@@ -1,7 +1,11 @@
-"""Instruction-for-instruction comparison of every kernel in two cubins (no GPU needed).
+r"""Instruction-for-instruction comparison of every kernel in two cubins (no GPU needed).
 
-Usage: sass_compare.py OLD.cubin NEW.cubin
+Usage: sass_compare.py [--map PATTERN=REPLACEMENT ...] OLD.cubin NEW.cubin
 (cubins from nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -cubin ...)
+
+Kernels are paired by demangled name.  --map rewrites NEW's demangled names (Python re.sub) before pairing, so that a kernel
+that gained a template argument meets its old self, e.g. --map 'k_analyse<(\d+), (\w+), (\w+), false>=k_analyse<\1, \2, \3>';
+with --map, a kernel only in NEW is reported as ADDED and is not an error.
 
 For every kernel symbol of either cubin it prints one of
   identical      the same instruction stream
@@ -10,6 +14,7 @@ For every kernel symbol of either cubin it prints one of
                  counts as one hex immediate
   DIFFERENT      anything else, with the first differing instruction
   MISSING        the symbol is in one cubin only
+  ADDED          (with --map) the symbol is in NEW only
 and exits with status 1 if any kernel is DIFFERENT or MISSING."""
 import os
 import re
@@ -79,19 +84,34 @@ def compare(a, b):
 
 
 def main():
-    if len(sys.argv) != 3:
+    args, maps = sys.argv[1:], []
+    while len(args) >= 2 and args[0] == "--map" and "=" in args[1]:
+        maps.append(args[1].split("=", 1))
+        args = args[2:]
+    if len(args) != 2:
         sys.exit(__doc__)
-    old, new = kernels(sys.argv[1]), kernels(sys.argv[2])
-    names = sorted(set(old) | set(new))
-    pretty = demangle(names)
+    old, new = kernels(args[0]), kernels(args[1])
+    pretty = demangle(sorted(set(old) | set(new)))
+    old = {pretty[n]: v for n, v in old.items()}
+    renamed = {}
+    for n, v in new.items():
+        name = pretty[n]
+        for pat, rep in maps:
+            name = re.sub(pat, rep, name)
+        renamed[name] = (v, pretty[n])
     bad = False
-    for n in names:
-        if n not in old or n not in new:
-            verdict, detail = "MISSING", "only in " + ("NEW" if n not in old else "OLD")
+    for name in sorted(set(old) | set(renamed)):
+        if name not in renamed:
+            verdict, detail = "MISSING", "only in OLD"
+        elif name not in old:
+            verdict, detail = ("ADDED", "") if maps else ("MISSING", "only in NEW")
         else:
-            verdict, detail = compare(old[n], new[n])
+            verdict, detail = compare(old[name], renamed[name][0])
         bad = bad or verdict in ("DIFFERENT", "MISSING")
-        print(f"{verdict:<10} {pretty[n]}" + (f": {detail}" if detail else ""))
+        label = name
+        if name in renamed and renamed[name][1] != name:
+            label = f"{name} -> {renamed[name][1]}" if name in old else renamed[name][1]
+        print(f"{verdict:<10} {label}" + (f": {detail}" if detail else ""))
     sys.exit(1 if bad else 0)
 
 
